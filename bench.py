@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the decoder hot path (BASELINE.json metric: decoder audio-seconds per second).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = Decoder.forward over one synthetic batch of BASELINE.json configs[1]
 (hifigan, B=64 utterances x 5 s = T 200 frames, random-init weights, bf16 tensor-core path).
@@ -25,6 +25,10 @@ decoder through PyTorch eager on the same GPU, fp32 and bf16 autocast: the pre-e
             under baseline/_ref (oracle/stage_reference.py; kind "reference"), else the torch-CPU port (kind "port")
 
 --impl reference times that same CPU arm on a bounded sample of the workload (8 utterances per step).
+
+--dump-outputs DIR writes the waveforms of the last timed step (gathered on rank 0 for N>1) as DIR/waveform.npy, float32
+[utterances, 1, samples], so that two builds run with the same arguments (hence the same inputs, weights and noise seeds)
+can be compared output for output.  Above 64 MiB it keeps a fixed, seeded sample of the utterances.
 """
 from __future__ import annotations
 
@@ -62,7 +66,13 @@ def parse():
                     help="N > 1: NCCL send / recv on a side stream (default), or decode straight into rank 0's buffer over NVLink "
                          "(symmetric memory; bit-identical, measured 1-2 %% slower per step at N = 2: the last kernel's stores go remote)")
     ap.add_argument("--no-aux", action="store_true", help="skip every auxiliary measurement (cfg3/cfg4/cfg5/eager_gpu)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the waveforms of the last timed step to DIR/waveform.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 path computes; it does not apply to --impl reference")
+    return a
 
 
 def workload_config(a, n_gpus):
@@ -138,7 +148,7 @@ def run_reference(a, rank, world):
     if rank != 0:
         return None
     frames = a.cpu_frames or a.frames
-    steps, warmup = max(1, min(a.steps, 5)), max(1, min(a.warmup, 1))
+    steps, warmup = a.steps, max(1, min(a.warmup, 1))
     r = cpu_reference_run(a.variant, frames, steps, warmup, batch=a.cpu_batch)
     line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": a.gpus, "steps": steps,
             "warmup": warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "weak",
@@ -408,6 +418,24 @@ def aux_cfg4(torch, dist, m, dev, rank, world, precision, direct=True):
                        "tail after the last forward (exposed_gather_tail_ms) is not hidden"}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_waveform(out_dir, wave):
+    """DIR/waveform.npy: float32 [B,1,S]; above DUMP_BYTES, a seeded sample of utterances (and of leading samples if a single
+    utterance is larger), the same one for the same arguments."""
+    import numpy as np
+    import torch
+    n, row_bytes = wave.shape[0], wave[0].numel() * 4
+    keep = max(1, min(n, DUMP_BYTES // row_bytes))
+    if keep < n:
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        wave = wave[torch.from_numpy(rows).to(wave.device)]
+    wave = wave[..., :DUMP_BYTES // 4]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "waveform.npy"), wave.float().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------
 # B200 arm
 # ------------------------------------------------------------------------------------------------
@@ -482,10 +510,11 @@ def run_b200(a, rank, local_rank, world):
         barrier()
         evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         t_wall = time.perf_counter()
+        out = None
         for i in range(steps):
             flush.fill_(i & 0xFF)                    # L2 flush, outside the event pair
             evs[i][0].record()
-            fn(warmup + i)
+            out = fn(warmup + i)
             if gatherer is not None and i == steps - 1:
                 gatherer.finish()                    # every gather of the timed steps completes inside the last event pair
             evs[i][1].record()
@@ -495,14 +524,21 @@ def run_b200(a, rank, local_rank, world):
         total = torch.tensor([sum(ms)], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(total, op=dist.ReduceOp.MAX)
-        return float(total.item()), ms, wall
+        return float(total.item()), ms, wall, out
 
     sampler = ClockSampler(local_rank)
     sampler.start()
-    total_ms, per_step, wall = timed(step_resident, a.steps, a.warmup)
+    total_ms, per_step, wall, last = timed(step_resident, a.steps, a.warmup)
     clocks = sampler.summary()
     sampler.stop()
     launches = m.last_launch_count()
+    if a.dump_outputs:
+        # what a caller of the timed path holds after its last step: N > 1 gathers every rank's waveforms on rank 0
+        wave = gatherer.finish() if gatherer is not None else last
+        if rank == 0:
+            dump_waveform(a.dump_outputs, wave)
+        barrier()                                    # no rank writes into rank 0's buffer again before it is read
+    last = None
     run_e2e(max(2, a.warmup // 2 + 1), 4000)                  # warm-up
     barrier()
     t_e2e = time.perf_counter()                                # host clock: the loop ends with every waveform on the host

@@ -89,7 +89,7 @@ def adain_resblock1(W, name, x, s, k, dil=(1, 3, 5), taps=None):
 def source_module(W, f0_curve, scale, noise):
     """SineGen + SourceModuleHnNSF, hifigan.py:117-157, 189-218, 254-264 (noise = the randn_like draw)."""
     f0 = F.interpolate(f0_curve[:, None], scale_factor=float(scale), mode="nearest").transpose(1, 2)   # [B,S,1]
-    fn = f0 * torch.arange(1, 10, dtype=torch.float32).view(1, 1, 9)
+    fn = f0 * torch.arange(1, 10, dtype=torch.float32, device=f0.device).view(1, 1, 9)
     rad = (fn / 24000) % 1
     rad = F.interpolate(rad.transpose(1, 2), scale_factor=1 / scale, mode="linear").transpose(1, 2)
     phase = torch.cumsum(rad, dim=1) * 2 * np.pi

@@ -523,6 +523,25 @@ def test_two_devices_in_one_process():
     assert torch.isfinite(outs[0]).all() and torch.equal(outs[0], outs[1])
 
 
+def test_torch_port_on_the_gpu_matches_golden():
+    """bench.py's eager_gpu leg runs oracle/decoder_torch.py on the GPU when the unmodified reference modules are not staged:
+    on CUDA tensors (TF32 off) it reproduces the reference waveforms it is pinned to on the host."""
+    from oracle import decoder_torch as OT
+    tf32 = torch.backends.cudnn.allow_tf32
+    torch.backends.cudnn.allow_tf32 = False
+    try:
+        for cfg, name, seed in ((DecoderConfig.hifigan(), "hifigan_B2_T5_w0_i1001.npz", 1001),
+                                (DecoderConfig.istftnet(), "istftnet_B2_T5_w0_i1005.npz", 1005)):
+            W = OT.TorchWeights({k: v.cuda() for k, v in synth.make_state_dict(cfg, 0, True).items()})
+            t = {k: v.cuda() for k, v in synth.make_inputs(2, 5, seed, cfg).items()}
+            out = OT.decoder_forward(W, cfg, t["asr"], t["F0_curve"], t["N"], t["s"], t["noise"]).cpu().numpy()
+            err = float(np.abs(out - golden(name)["out"]).max())
+            G.log("torch_port_gpu_vs_golden", fixture=name, maxabs=err)
+            assert err <= 1e-3, (name, err)
+    finally:
+        torch.backends.cudnn.allow_tf32 = tf32
+
+
 # ---------------------------------------------------------------- §8(f) N4: the Vocos decoder variant (Modules/vocos.py)
 def _vocos_inputs(B, T, seed, cfg):
     return {k: v.numpy() for k, v in synth.make_inputs(B, T, seed, cfg, with_noise=False).items()}
