@@ -312,6 +312,20 @@ ST2_API int st2_adain_conv1d_row(const float* x, const float* h, const float* al
                          void* scratch, int32_t B, int32_t T, int32_t C, int32_t k, int32_t padding, int32_t dilation,
                          float scale, int32_t precision, int32_t x16, int32_t y16, void* stream);
 
+/* Two chained half-steps on the row-per-thread kernel, as one iteration of AdaINResBlock1 (Modules/hifigan.py:67-73) runs them
+ * in the decoder (x stored as fp16, padding dil * (k - 1) / 2):
+ *   y1 = conv1d(snake(AdaIN(x; h1), alpha1), w1) + bias1                    (stored as fp16)
+ *   y2 = conv1d(snake(AdaIN(y1; h2), alpha2), w2) + bias2 + x                (stored as fp16)
+ * The second launch computes the AdaIN coefficients of y1 itself from the statistics partials of the first when its table of
+ * them fits (<= 2 KB per CTA, and switch "no_row_inline_coef" off); otherwise the coefficient kernel runs between the two.
+ * *inline_coef (host, may be NULL) receives 1 if the second launch computed them itself.  y1 / y2 [B,T,C] fp32 receive the
+ * stored fp16 values widened; if h_next is given, coef_next [B,2,C] the AdaIN coefficients of y2. */
+ST2_API int64_t st2_adain_conv1d_row_pair_scratch_bytes(int32_t B, int32_t T, int32_t C, int32_t k1, int32_t k2);
+ST2_API int st2_adain_conv1d_row_pair(const float* x, const float* h1, const float* alpha1, const float* w1, const float* bias1,
+                              const float* h2, const float* alpha2, const float* w2, const float* bias2, float* y1, float* y2,
+                              const float* h_next, float* coef_next, int32_t* inline_coef, void* scratch, int32_t B, int32_t T,
+                              int32_t C, int32_t k1, int32_t dil1, int32_t k2, int32_t dil2, int32_t precision, void* stream);
+
 /* Generator upsampling step (Modules/hifigan.py:329-334) through the fused tensor-core kernels:
  *   y = conv_transpose1d(act(x), w) + bias + res        x [B,Tin,Cin], w [Cin,Cout,k] (k a multiple of stride),
  * res / y [B,Tout,Cout], Tout = (Tin-1)*stride - 2*padding + k + output_padding.  alpha [Cin] for snake.

@@ -111,6 +111,9 @@ SIGNATURES = {
     "st2_adain_conv1d_row_scratch_bytes": (_L, [_I, _I, _I, _I]),
     "st2_adain_conv1d_row": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, C.c_float, _I, _I, _I,
                                        _P]),
+    "st2_adain_conv1d_row_pair_scratch_bytes": (_L, [_I, _I, _I, _I, _I]),
+    "st2_adain_conv1d_row_pair": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.POINTER(_I), _P, _I, _I, _I, _I,
+                                            _I, _I, _I, _I, _P]),
     "st2_act_conv_transpose1d_fused_scratch_bytes": (_L, [_I, _I, _I, _I, _I, _I]),
     "st2_act_conv_transpose1d_fused": (C.c_int, [_P, _P, _I, C.c_float, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I,
                                                  _I, _P]),
@@ -144,6 +147,22 @@ def check(status: int, what: str = "") -> int:
         msg = load().st2_last_error()
         raise St2Error("%s failed (%d): %s" % (what or "st2 call", status, msg.decode() if msg else ""))
     return status
+
+
+_tuning_generation = 0
+
+
+def set_tuning(name: str, value: int) -> None:
+    """st2_set_tuning (a process-wide kernel-selection / planner switch), noted in tuning_generation() so that decoder modules
+    plan their workspace and capture their CUDA graphs again instead of reusing what the old switches produced."""
+    global _tuning_generation
+    check(load().st2_set_tuning(name.encode(), int(value)), "st2_set_tuning(%s)" % name)
+    _tuning_generation += 1
+
+
+def tuning_generation() -> int:
+    """How many times set_tuning() has changed a switch in this process."""
+    return _tuning_generation
 
 
 def ptr(t) -> C.c_void_p:

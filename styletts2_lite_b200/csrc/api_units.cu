@@ -289,6 +289,104 @@ int st2_adain_conv1d_row(const float* x, const float* h, const float* alpha, con
     return e;
 }
 
+// Two chained half-steps on conv_row.cu as one iteration of AdaINResBlock1 runs them in the decoder: the second launch reads the
+// first one's fp16 output and, when its coefficient table fits, computes that output's AdaIN coefficients itself from the
+// first launch's statistics partials (RowCoefSrc) instead of from a coefficient launch in between.
+static int64_t row_pair_offsets(int B, int T, int C, int k1, int k2, int64_t off[13]) {
+    int64_t o = 0;
+    off[0] = o; o += align256((int64_t)k1 * C * C * sizeof(float));              // packed fp32 weights of step 1
+    off[1] = o; o += align256((int64_t)k1 * 64 * C * 2);                         // 16-bit weights of step 1
+    off[2] = o; o += align256((int64_t)k2 * C * C * sizeof(float));              // step 2
+    off[3] = o; o += align256((int64_t)k2 * 64 * C * 2);
+    off[4] = o; o += align256(adain_scratch_bytes(B, T, C));                     // statistics of x
+    off[5] = o; o += align256((int64_t)B * 2 * C * sizeof(float));               // coefficients of x
+    off[6] = o; o += align256((int64_t)B * 2 * C * sizeof(float));               // coefficients of y1 (coefficient-kernel path)
+    off[7] = o; o += align256(conv_row_stats_bytes(B, T, C));                    // partials of y1
+    off[8] = o; o += align256(conv_row_stats_bytes(B, T, C));                    // partials of y2
+    off[9] = o; o += align256((int64_t)B * T * C * 2);                           // x as fp16
+    off[10] = o; o += align256((int64_t)B * T * C * 2);                          // y1 as fp16
+    off[11] = o; o += align256((int64_t)B * T * C * 2);                          // y2 as fp16
+    off[12] = o;
+    return o;
+}
+
+int64_t st2_adain_conv1d_row_pair_scratch_bytes(int32_t B, int32_t T, int32_t C, int32_t k1, int32_t k2) {
+    if (B <= 0 || T <= 0 || !(C == 32 || C == 64) || k1 <= 0 || k2 <= 0) return ST2_ERR_INVALID;
+    int64_t off[13];
+    return row_pair_offsets(B, T, C, k1, k2, off);
+}
+
+int st2_adain_conv1d_row_pair(const float* x, const float* h1, const float* alpha1, const float* w1, const float* bias1,
+                              const float* h2, const float* alpha2, const float* w2, const float* bias2, float* y1, float* y2,
+                              const float* h_next, float* coef_next, int32_t* inline_coef, void* scratch, int32_t B, int32_t T,
+                              int32_t C, int32_t k1, int32_t dil1, int32_t k2, int32_t dil2, int32_t precision, void* stream) {
+    ST2_REQUIRE(x && h1 && alpha1 && w1 && h2 && alpha2 && w2 && y1 && y2 && scratch && B > 0 && T > 0 && (C == 32 || C == 64) &&
+                    k1 > 0 && k2 > 0 && dil1 > 0 && dil2 > 0,
+                "adain_conv1d_row_pair: bad argument");
+    ST2_REQUIRE(precision == ST2_PREC_BF16 || precision == ST2_PREC_FP16, "adain_conv1d_row_pair: 16-bit precisions only");
+    ST2_REQUIRE(dil1 * (k1 - 1) % 2 == 0 && dil2 * (k2 - 1) % 2 == 0, "adain_conv1d_row_pair: length-preserving convolutions only");
+    ST2_REQUIRE((h_next == nullptr) == (coef_next == nullptr), "adain_conv1d_row_pair: h_next and coef_next go together");
+    cudaStream_t st = (cudaStream_t)stream;
+    int64_t off[13];
+    row_pair_offsets(B, T, C, k1, k2, off);
+    char* base = (char*)scratch;
+    float* wp1 = (float*)(base + off[0]);
+    void* w16_1 = base + off[1];
+    float* wp2 = (float*)(base + off[2]);
+    void* w16_2 = base + off[3];
+    void* xstats = base + off[4];
+    float* coef1 = (float*)(base + off[5]);
+    float* coef2 = (float*)(base + off[6]);
+    void* parts1 = base + off[7];
+    void* parts2 = base + off[8];
+    void* x16b = base + off[9];
+    void* y1_16 = base + off[10];
+    void* y2_16 = base + off[11];
+    const int dt = precision == ST2_PREC_BF16 ? DT_BF16 : DT_F16;
+    const int64_t n = (int64_t)B * T * C;
+    int e = launch_fold_pack(nullptr, w1, wp1, C, C, k1, 0, st);
+    if (e == ST2_OK) e = launch_pack_w16(wp1, w16_1, k1, C, C, 64, C, dt, st);
+    if (e == ST2_OK) e = launch_fold_pack(nullptr, w2, wp2, C, C, k2, 0, st);
+    if (e == ST2_OK) e = launch_pack_w16(wp2, w16_2, k2, C, C, 64, C, dt, st);
+    if (e == ST2_OK) e = launch_in_stats(x, C, B, T, C, xstats, st);
+    if (e == ST2_OK) e = launch_adain_coef(xstats, h1, 2 * C, 0, coef1, B, T, C, C, st);
+    if (e == ST2_OK) e = launch_cast16(x, x16b, n, DT_F16, st);
+    if (e != ST2_OK) return e;
+    ConvArgs a1;
+    memset(&a1, 0, sizeof(a1));
+    a1.B = B; a1.Cin = C; a1.Cout = C; a1.Tin = T; a1.Tout = T; a1.M = T;
+    a1.x = (const float*)x16b; a1.ld_x = C; a1.x16in = 1;
+    a1.w = wp1; a1.w16 = w16_1; a1.w16_cin_pad = 64; a1.w16_cout_pad = C; a1.fmt16 = dt;
+    a1.bias = bias1;
+    a1.y = (float*)y1_16; a1.ld_y = C; a1.y16out = 1;
+    a1.ntaps = k1; a1.tap_step = dil1; a1.in_off = -dil1 * (k1 - 1) / 2; a1.in_stride = 1;
+    a1.phases = 1; a1.w_step = 1; a1.out_stride = 1; a1.out_pad = 0;
+    a1.scale = 1.f;
+    ConvArgs a2 = a1;                              // y2 = conv(snake(AdaIN(y1))) + bias2 + x
+    a2.x = (const float*)y1_16;
+    a2.w = wp2; a2.w16 = w16_2;
+    a2.bias = bias2;
+    a2.res = (const float*)x16b; a2.ld_res = C; a2.res16 = 1;
+    a2.y = (float*)y2_16;
+    a2.ntaps = k2; a2.tap_step = dil2; a2.in_off = -dil2 * (k2 - 1) / 2;
+    ST2_REQUIRE(conv_row_can_launch(a1) && conv_row_can_launch(a2), "adain_conv1d_row_pair: geometry not supported by conv_row");
+    RowStatsDesc rd1, rd2;
+    e = launch_conv_row(a1, coef1, C, ACT_SNAKE, alpha1, parts1, &rd1, st);
+    if (e != ST2_OK) return e;
+    const bool inl = conv_row_inline_coef_ok(a2);
+    if (inline_coef != nullptr) *inline_coef = inl ? 1 : 0;
+    const RowCoefSrc src{parts1, rd1, h2, 2 * C, 0, T};
+    if (!inl) {
+        e = launch_adain_coef_row(parts1, rd1, h2, 2 * C, 0, coef2, B, T, C, C, st);
+        if (e != ST2_OK) return e;
+    }
+    e = launch_conv_row(a2, coef2, C, ACT_SNAKE, alpha2, h_next ? parts2 : nullptr, &rd2, st, inl ? &src : nullptr);
+    if (e == ST2_OK) e = launch_half_to_float(y1_16, y1, n, st);
+    if (e == ST2_OK) e = launch_half_to_float(y2_16, y2, n, st);
+    if (e == ST2_OK && h_next != nullptr) e = launch_adain_coef_row(parts2, rd2, h_next, 2 * C, 0, coef_next, B, T, C, C, st);
+    return e;
+}
+
 // Generator upsampling step (hifigan.py:329-334): y = conv_transpose1d(act(x), w) + bias + res, plus the AdaIN
 // coefficients of y for style h_next, through the fused tensor-core kernels.
 static int64_t fused_t_offsets(int B, int Tin, int Cin, int Cout, int k, int stride, int64_t off[5]) {

@@ -57,6 +57,7 @@ struct Tune {
     int no_row_bias_mma = 0;                // conv_row: bias added in the epilogue everywhere (A/B of the bias MMA)
     int no_row_inline_coef = 0;             // conv_row: always launch the coefficient kernel (A/B of the in-kernel coefficients)
     int row_sub = 0, row_slot = 0, row_na = 0;                  // conv_row planner overrides for sweeps (0 = planner's choice)
+    int row_always = 0;                     // conv_row: take every geometry it can launch, small problems too (tests of its scheduling)
     int no_xt16 = 0, no_run16 = 0, no_xu16 = 0, no_sum16 = 0;   // defaults of the per-handle storage options (st2_decoder_set_option)
     int no_src16 = 0, no_out16 = 0;
 };

@@ -767,14 +767,15 @@ bool conv_row_can_launch(const ConvArgs& a) {
 }
 
 // dispatch policy: small problems (one-sentence latency: fewer than 4 macro tiles per SM) stay on conv_pipe.cu, whose 128-row
-// tiles spread them over more SMs
+// tiles spread them over more SMs.  Tune::row_always drops that threshold (geometry and plan still apply), so the decoder's
+// reference fixtures, a few utterances long, can run every 32 / 64-channel resblock conv on this kernel.
 bool conv_row_supported(const ConvArgs& a) {
     if (row_disabled() || !row_geometry_ok(a)) return false;
     RowParams p;
     size_t smem;
     int grid;
     if (!row_plan(a, p, &smem, &grid)) return false;
-    return (int64_t)a.B * p.mmt >= 4 * (int64_t)row_num_sms();
+    return tune().row_always || (int64_t)a.B * p.mmt >= 4 * (int64_t)row_num_sms();
 }
 
 // bytes of the statistics buffer a conv_row launch of this geometry writes (upper bound over devices with <= RW_MAXGRID SMs)
@@ -844,8 +845,9 @@ int launch_conv_row(const ConvArgs& a, const float* coef, int coef_ld, int act, 
         desc->grid = grid; desc->J = p.J; desc->nwarp = 4 * nch; desc->mmt = p.mmt; desc->tq = p.tq; desc->tr = p.tr; desc->C = C;
     }
     if (tune().verbose)
-        fprintf(stderr, "conv_row: C=%d taps=%d step=%d x16=%d y16=%d nres=%d sub=%d R=%d nblk=%d tail=%d na=%d lw=%d xd=%d nr=%d smem=%zu grid=%d tq=%d J=%d\n",
-                C, p.ntaps, p.tap_step, a.x16in, a.y16out, p.nres, p.sub, p.R, p.nblk, p.tail_rows, p.na, p.lw, p.xd, p.nr, smem, grid, p.tq, p.J);
+        fprintf(stderr, "conv_row: C=%d taps=%d step=%d x16=%d y16=%d nres=%d sub=%d R=%d nblk=%d tail=%d na=%d lw=%d xd=%d nr=%d smem=%zu grid=%d mmt=%d tq=%d tr=%d J=%d inline=%d\n",
+                C, p.ntaps, p.tap_step, a.x16in, a.y16out, p.nres, p.sub, p.R, p.nblk, p.tail_rows, p.na, p.lw, p.xd, p.nr, smem, grid, p.mmt,
+                p.tq, p.tr, p.J, p.cin_part != nullptr ? 1 : 0);
     ST2_REQUIRE(stats_out == nullptr || (int64_t)grid * p.J * (4 * nch) * 32 * 8 <= conv_row_stats_bytes(a.B, a.Tout, C),
                 "conv_row: statistics buffer too small");
     // the opt-in to > 48 KB of dynamic shared memory is per device: once per (device, variant)

@@ -435,7 +435,8 @@ const TuneField kTuneFields[] = {
     {"no_run16", "ST2_NO_RUN16", &Tune::no_run16, true}, {"no_xu16", "ST2_NO_XU16", &Tune::no_xu16, true},
     {"no_sum16", "ST2_NO_SUM16", &Tune::no_sum16, true}, {"no_src16", "ST2_NO_SRC16", &Tune::no_src16, true},
     {"no_out16", "ST2_NO_OUT16", &Tune::no_out16, true}, {"row_sub", "ST2_ROW_SUB", &Tune::row_sub, false},
-    {"row_slot", "ST2_ROW_SLOT", &Tune::row_slot, false}, {"row_na", "ST2_ROW_NA", &Tune::row_na, false}};
+    {"row_slot", "ST2_ROW_SLOT", &Tune::row_slot, false}, {"row_na", "ST2_ROW_NA", &Tune::row_na, false},
+    {"row_always", "ST2_ROW_ALWAYS", &Tune::row_always, true}};
 Tune& tune_storage() {
     static Tune t = [] {
         Tune v;

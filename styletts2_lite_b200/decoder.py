@@ -62,7 +62,8 @@ class B200Decoder(nn.Module):
         self._taps: Dict[str, torch.Tensor] = {}
         self._graphs: "collections.OrderedDict[tuple, dict]" = collections.OrderedDict()   # LRU: newest last
         self.max_graphs = 8                     # each captured shape owns a private workspace + static I/O: bound the cache
-        self._ws_bytes: Dict[tuple, int] = {}   # (B, T, precision) -> workspace bytes (the host dry run costs ~0.1 ms)
+        self._ws_bytes: Dict[tuple, int] = {}   # (B, T, precision, plan) -> workspace bytes (the host dry run costs ~0.1 ms)
+        self._option_generation = 0             # bumped by set_option(): part of the plan key of both caches
         self._profiling = False
         self.train(False)
 
@@ -110,6 +111,18 @@ class B200Decoder(nn.Module):
     def num_params(self) -> int:
         return sum(p.numel() for p in self.parameters())
 
+    def set_option(self, name: str, value: int) -> None:
+        """st2_decoder_set_option on this module's handle ("fp16_xt", "fp16_run", ...: INTEGRATION.md section 3e).  The next
+        forward plans its workspace and captures its CUDA graph again."""
+        if self._handle is None:
+            self._sync(next(self.parameters()).device)
+        _lib.check(_lib.load().st2_decoder_set_option(self._handle, name.encode(), int(value)), "set_option(%s)" % name)
+        self._option_generation += 1
+
+    def _plan_key(self) -> tuple:
+        # the switches that decide the kernel plan, and with it the workspace size and the launches a graph captures
+        return (_lib.tuning_generation(), self._option_generation)
+
     # ---- forward ---------------------------------------------------------------------------
     def workspace_bytes(self, B: int, T: int, precision: Optional[str] = None) -> int:
         lib = _lib.load()
@@ -133,14 +146,14 @@ class B200Decoder(nn.Module):
 
     # ---- CUDA-graph replay for small batches ------------------------------------------------
     def _forward_graph(self, asr, F0_curve, N, s, seed, prec_name):
-        """One captured graph per (B, T, precision, device): the ~270 launches of a forward replay as one graph launch.
-        Inputs are copied into the graph's static buffers, the Philox seed lives in device memory
+        """One captured graph per (B, T, precision, device, switches): the ~270 launches of a forward replay as one graph
+        launch.  Inputs are copied into the graph's static buffers, the Philox seed lives in device memory
         (st2_decoder_set_seed_buffer), the returned waveform is a copy of the static output."""
         lib = _lib.load()
         dev = asr.device
         B, _, T = asr.shape
         prec = _lib.PREC[prec_name]
-        key = (B, T, prec, dev.index)
+        key = (B, T, prec, dev.index) + self._plan_key()
         g = self._graphs.get(key)
         if g is not None:
             self._graphs.move_to_end(key)
@@ -233,7 +246,7 @@ class B200Decoder(nn.Module):
         return out
 
     def _workspace_need(self, B: int, T: int, prec: int) -> int:
-        key = (B, T, prec)
+        key = (B, T, prec) + self._plan_key()
         n = self._ws_bytes.get(key)
         if n is None:
             n = _lib.check(_lib.load().st2_decoder_workspace_bytes(self._handle, B, T, prec), "st2_decoder_workspace_bytes")

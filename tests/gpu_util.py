@@ -162,6 +162,32 @@ def adain_conv1d_row(x_btc, h, alpha, w, bias, res_btc, old_btc, h_next, padding
     return y.cpu().numpy(), (None if cn is None else cn.cpu().numpy())
 
 
+def adain_conv1d_row_pair(x_btc, h1, alpha1, w1, b1, h2, alpha2, w2, b2, h_next, dil1, dil2, precision="bf16"):
+    """Two chained half-steps on conv_row.cu (y1 = step(x), y2 = step(y1) + x, x stored as fp16); returns
+    (y1, y2, coef_next, inline) with y1 / y2 channels-last [B,T,C] and `inline` whether the second launch computed the AdaIN
+    coefficients of y1 itself."""
+    lib = _lib.load()
+    B, T, Cc = x_btc.shape
+    k1, k2 = w1.shape[2], w2.shape[2]
+    xd, h1d, a1d, w1d = to_dev(x_btc), to_dev(h1), to_dev(alpha1.reshape(-1)), to_dev(w1)
+    h2d, a2d, w2d = to_dev(h2), to_dev(alpha2.reshape(-1)), to_dev(w2)
+    b1d = None if b1 is None else to_dev(b1)
+    b2d = None if b2 is None else to_dev(b2)
+    hn = None if h_next is None else to_dev(h_next)
+    cn = None if h_next is None else torch.full((B, 2, Cc), float("nan"), device=dev())
+    y1 = torch.full((B, T, Cc), float("nan"), device=dev())
+    y2 = torch.full((B, T, Cc), float("nan"), device=dev())
+    inline = C.c_int32(-1)
+    nbytes = _lib.check(lib.st2_adain_conv1d_row_pair_scratch_bytes(B, T, Cc, k1, k2), "row_pair_scratch_bytes")
+    scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev())
+    _lib.check(lib.st2_adain_conv1d_row_pair(_lib.ptr(xd), _lib.ptr(h1d), _lib.ptr(a1d), _lib.ptr(w1d), _lib.ptr(b1d),
+                                             _lib.ptr(h2d), _lib.ptr(a2d), _lib.ptr(w2d), _lib.ptr(b2d), _lib.ptr(y1), _lib.ptr(y2),
+                                             _lib.ptr(hn), _lib.ptr(cn), C.byref(inline), _lib.ptr(scratch), B, T, Cc, k1, dil1,
+                                             k2, dil2, _lib.PREC[precision], stream()), "adain_conv1d_row_pair")
+    torch.cuda.synchronize()
+    return y1.cpu().numpy(), y2.cpu().numpy(), (None if cn is None else cn.cpu().numpy()), inline.value == 1
+
+
 def act_conv_transpose1d_fused(x_btc, alpha, act, w, bias, res_btc, h_next, stride, padding, output_padding, slope=0.0,
                                precision="bf16"):
     """Fused upsampling step on channels-last tensors; returns (y [B,Tout,Cout], coef_next [B,2,Cout] or None)."""

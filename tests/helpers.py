@@ -26,6 +26,24 @@ def golden(name):
     return np.load(os.path.join(GOLDEN, name))
 
 
+def resblock_tap_shapes(T, stages=range(4)):
+    """{tap name: (rows, C)} of the HiFi-GAN generator's AdaINResBlock1 layers in `stages`: every conv1 output (`.convs1.j`),
+    every running tensor (`.iterj`; the last one of a resblock is folded into the stage sum) and every stage input / output,
+    for an utterance of T asr frames.  The names are the taps of oracle/decoder_torch.py and of B200Decoder.set_tap."""
+    lens = [20 * T, 100 * T, 300 * T, 600 * T]
+    names = {}
+    for i in stages:
+        C_ = 256 >> i
+        names["generator.stage%d.in" % i] = (lens[i], C_)
+        names["generator.stage%d.out" % i] = (lens[i], C_)
+        for blk in ["generator.noise_res.%d" % i] + ["generator.resblocks.%d" % (3 * i + j) for j in range(3)]:
+            for j in range(3):
+                names["%s.convs1.%d" % (blk, j)] = (lens[i], C_)
+                if j < 2 or "noise_res" in blk:
+                    names["%s.iter%d" % (blk, j)] = (lens[i], C_)
+    return names
+
+
 def snr_db(ref, x):
     ref = ref.astype(np.float64)
     err = x.astype(np.float64) - ref

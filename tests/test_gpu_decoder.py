@@ -10,7 +10,7 @@ import torch
 from styletts2_lite_b200.config import DecoderConfig
 from styletts2_lite_b200 import synth
 from oracle import decoder_np as O
-from helpers import golden, np_inputs, np_state_dict, rel_l2, snr_db
+from helpers import golden, np_inputs, np_state_dict, rel_l2, resblock_tap_shapes, snr_db
 
 pytestmark = pytest.mark.gpu
 
@@ -423,16 +423,7 @@ def test_bf16_every_resblock_tap_at_3s():
     m = _decoder(cfg)
     inp = np_inputs(1, T, 1001, cfg)
     names = {"encode": (T, 1024), "decode.0": (T, 1024), "decode.3": (2 * T, 512)}
-    lens = [20 * T, 100 * T, 300 * T, 600 * T]
-    for i in range(4):
-        C_ = 256 >> i
-        names["generator.stage%d.in" % i] = (lens[i], C_)
-        names["generator.stage%d.out" % i] = (lens[i], C_)
-        for blk in ["generator.noise_res.%d" % i] + ["generator.resblocks.%d" % (3 * i + j) for j in range(3)]:
-            for j in range(3):
-                names["%s.convs1.%d" % (blk, j)] = (lens[i], C_)
-                if j < 2 or "noise_res" in blk:
-                    names["%s.iter%d" % (blk, j)] = (lens[i], C_)
+    names.update(resblock_tap_shapes(T))
     bufs = {n: m.set_tap(n, 1, rows, C_) for n, (rows, C_) in names.items()}
     out = _run(m, inp, precision="bf16")
     taps = {}
