@@ -128,10 +128,8 @@ ST2_API int st2_decoder_set_tap(st2_decoder* d, const char* name, float* dst, in
  * "fp16_xu", "fp16_sum" (default 1 each) switch the four kinds of tensors individually.  Unknown names fail. */
 ST2_API int st2_decoder_set_option(st2_decoder* d, const char* name, int32_t value);
 
-/* Process-wide kernel-selection / planner switches for A/B measurements and for testing a fallback kernel ("no_pipe", "no_row",
- * "no_fused", "no_pdl", "pipe_xmax", ...; the full list is kTuneFields in csrc/decoder.cu).  Each is initialised ONCE from the
- * environment variable ST2_<NAME> when the library first needs it; this call is the only other way to change one -- nothing
- * on the forward path reads the environment.  Not synchronised: call it while no forward is running.  Unknown names fail. */
+/* Process-wide test hooks: "no_pipe", "row_always", "row_sub", "no_row_inline_coef", "verbose" (default 0 each); unknown names
+ * fail.  Not synchronised: call it while no forward is running. */
 ST2_API int st2_set_tuning(const char* name, int32_t value);
 
 /* Optional device-resident Philox seed: when set (non-NULL), the harmonic source reads its noise seed from *dev_seed

@@ -50,9 +50,6 @@ def is_current() -> bool:
 
 
 def build(force: bool = False, verbose: bool = False) -> str:
-    # kernel-variant builds for A/B timing: ST2_BUILD_DEFINES="-DFOO" ST2_BUILD_OUT=libst2_foo.so python -m styletts2_lite_b200.build
-    if os.environ.get("ST2_BUILD_OUT"):
-        return _build_variant(os.environ.get("ST2_BUILD_DEFINES", "").split(), os.path.join(LIBDIR, os.environ["ST2_BUILD_OUT"]))
     if not force and is_current():
         return LIB
     os.makedirs(LIBDIR, exist_ok=True)
@@ -79,28 +76,6 @@ def build(force: bool = False, verbose: bool = False) -> str:
     with open(LIB + ".sha256", "w") as fh:
         fh.write(_digest())
     return LIB
-
-
-def _build_variant(defines, out):
-    os.makedirs(LIBDIR, exist_ok=True)
-    objdir = OBJDIR + "_" + os.path.basename(out)
-    os.makedirs(objdir, exist_ok=True)
-    nvcc = _nvcc()
-
-    def compile_one(src):
-        obj = os.path.join(objdir, src.replace(".cu", ".o"))
-        r = subprocess.run([nvcc] + NVCC_FLAGS + defines + ["-c", os.path.join(CSRC, src), "-o", obj], capture_output=True, text=True)
-        if r.returncode != 0:
-            raise RuntimeError("nvcc failed for %s:\n%s\n%s" % (src, r.stdout, r.stderr))
-        return obj
-
-    with ThreadPoolExecutor(max_workers=min(12, len(SOURCES))) as ex:
-        objs = list(ex.map(compile_one, SOURCES))
-    r = subprocess.run([nvcc, "-shared", "-o", out] + objs + ["-gencode", "arch=compute_100a,code=sm_100a", "-lcudart_static",
-                                                              "-Xcompiler", "-fPIC"], capture_output=True, text=True)
-    if r.returncode != 0:
-        raise RuntimeError("link failed:\n%s\n%s" % (r.stdout, r.stderr))
-    return out
 
 
 if __name__ == "__main__":

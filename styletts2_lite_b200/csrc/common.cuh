@@ -45,21 +45,14 @@ extern thread_local int64_t g_launch_count;
 
 static inline int cdiv(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 
-// Process-wide kernel-selection / planner switches (A/B experiments, tests of a fallback path).  They are read ONCE from the ST2_*
-// environment variables when first used -- so a sweep script can still set them per process -- and changed afterwards only
-// through st2_set_tuning(); nothing on the forward path calls getenv.  Not synchronised: set them while no forward is running.
+// Process-wide test hooks: they let the tests reach or pin a kernel path at fixture sizes.  All default to 0 (the planners'
+// choice) and are changed only through st2_set_tuning().  Not synchronised: set them while no forward is running.
 struct Tune {
-    int no_pdl = 0, pdl_always = 0, no_k32 = 0, no_xstage = 0, no_fused = 0;
-    int no_pipe = 0, no_pipe_ups = 0, no_pipe_nt = 0, no_pipe_pair = 0, no_row = 0;
-    int pipe_xmax = 0, pipe_xmax16 = 0, pipe_nacc = 0, pipe_eg3_nores = 0, pipe_eg = 0;
-    int pipe_nxg = 0, pipe_nrg = 0, pipe_na = 0, pipe_nx = 0, pipe_nr = 0;
-    int verbose = 0, tc_halo = 0, lstm_bt = 0;
-    int no_row_bias_mma = 0;                // conv_row: bias added in the epilogue everywhere (A/B of the bias MMA)
-    int no_row_inline_coef = 0;             // conv_row: always launch the coefficient kernel (A/B of the in-kernel coefficients)
-    int row_sub = 0, row_slot = 0, row_na = 0;                  // conv_row planner overrides for sweeps (0 = planner's choice)
+    int no_pipe = 0;                        // conv_pipe: decline every shape, so conv_fused runs the ones it would take
     int row_always = 0;                     // conv_row: take every geometry it can launch, small problems too (tests of its scheduling)
-    int no_xt16 = 0, no_run16 = 0, no_xu16 = 0, no_sum16 = 0;   // defaults of the per-handle storage options (st2_decoder_set_option)
-    int no_src16 = 0, no_out16 = 0;
+    int row_sub = 0;                        // conv_row: only this tile split (0 = planner's choice)
+    int no_row_inline_coef = 0;             // conv_row: always launch the coefficient kernel (reference for the in-kernel coefficients)
+    int verbose = 0;                        // print the conv_pipe / conv_row / lstm plans to stderr
 };
 const Tune& tune();
 int tune_set(const char* name, int value);    // ST2_OK, or ST2_ERR_INVALID for an unknown name

@@ -629,14 +629,14 @@ adain_coef_f2_kernel(const float2* __restrict__ partial, int nparts, const float
 int launch_adain_coef_f2(const void* partial, int nparts, const float* h, int ld_h, int h_off, float* coef, int B, int T,
                          int C, int Cpad, cudaStream_t st, const float* x_offset) {
     dim3 grid(cdiv(Cpad, 32), B);
-    // programmatic dependent launch for small grids (one-sentence latency; ST2_NO_PDL=1: plain): the CTAs may be scheduled while
-    // the producing conv drains.  Large batches gain nothing and lose SMs to the next conv's early CTAs (conv_pipe.cu)
+    // programmatic dependent launch for small grids (one-sentence latency): the CTAs may be scheduled while the producing conv
+    // drains.  Large batches gain nothing and lose SMs to the next conv's early CTAs (conv_pipe.cu)
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid; cfg.blockDim = dim3(1024); cfg.dynamicSmemBytes = 0; cfg.stream = st;
     cudaLaunchAttribute attr;
     attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr.val.programmaticStreamSerializationAllowed = 1;
-    const bool pdl = !tune().no_pdl && ((int64_t)grid.x * grid.y <= 64 || tune().pdl_always);
+    const bool pdl = (int64_t)grid.x * grid.y <= 64;
     cfg.attrs = &attr; cfg.numAttrs = pdl ? 1 : 0;
     ST2_CUDA_CHECK(cudaLaunchKernelEx(&cfg, adain_coef_f2_kernel, (const float2*)partial, nparts, h, ld_h, h_off, coef, T, C, Cpad, x_offset));
     ST2_LAUNCH_CHECK();
@@ -699,14 +699,14 @@ int launch_conv_fused(const ConvArgs& a, const float* coef, int coef_ld, int act
     p.stats = (float2*)stats_out;
     // shared-memory plan (one persistent CTA per SM, <= ~224 KB)
     const int64_t budget = 224 * 1024;
-    p.k32 = (a.Cin == 32 && a.w16_cin_pad == 64 && !tune().no_k32) ? 1 : 0;
+    p.k32 = (a.Cin == 32 && a.w16_cin_pad == 64) ? 1 : 0;
     const int64_t arow = p.k32 ? 64 : 128;
     const int64_t a_bytes = ((int64_t)p.rows * arow + 1023) & ~(int64_t)1023;
     const int64_t b_stage = (int64_t)bn * arow;
     const int64_t base_fixed = 2 * a_bytes + EW * 32 * 32 * 4 + (int64_t)EG * 4 * bn * 8 + 160 * 8 + 1024;
     // activations by TMA into an fp32 staging ring for single-chunk layers (C <= 64), when the ring fits
     const int64_t x_bytes = (((int64_t)p.rows * a.Cin * (a.x16in ? 2 : 4)) + 1023) & ~(int64_t)1023;
-    p.xstage = (p.kchunks == 1 && a.ld_x * (a.x16in ? 2 : 4) % 16 == 0 && !tune().no_xstage) ? 1 : 0;
+    p.xstage = (p.kchunks == 1 && a.ld_x * (a.x16in ? 2 : 4) % 16 == 0) ? 1 : 0;
     int64_t fixed = base_fixed + (p.xstage ? NSTG * x_bytes : 0);
     const int ktaps_total = a.phases > 1 ? a.ntaps * a.phases : a.ntaps;
     p.ktaps_total = ktaps_total;

@@ -811,7 +811,6 @@ static bool pipe_geometry_ok(const ConvArgs& a) {
         if (a.out_stride != a.phases || a.w_step != a.phases || a.tap_step != -1 || a.in_off != 0 || a.accumulate) return false;
         if (a.ld_y != a.Cout || (a.res != nullptr && a.ld_res != a.Cout)) return false;
         if (a.Tout % a.phases != 0 || a.out_pad < 0 || a.out_pad > a.phases) return false;
-        if (tune().no_pipe_ups) return false;
     } else if (a.out_stride != 1 || a.out_pad != 0 || a.tap_step <= 0 || a.M != a.Tout) {
         return false;
     }
@@ -821,7 +820,7 @@ static bool pipe_geometry_ok(const ConvArgs& a) {
         // tile that stays resident in the 4 operand buffers (<= 4 K chunks)
         const int ntot = a.phases * a.w16_cout_pad, kch = a.w16_cin_pad / 64;
         const bool one_pass = ntot <= 192;
-        const bool n_pass = ntot % 128 == 0 && ntot <= 1024 && (kch == 1 || kch == 2 || kch == 4) && !tune().no_pipe_nt;
+        const bool n_pass = ntot % 128 == 0 && ntot <= 1024 && (kch == 1 || kch == 2 || kch == 4);
         if (!one_pass && !n_pass) return false;
         // measured on the 256-channel layers (N passes here vs conv_fused.cu): k=3 0.278 -> 0.165 ms, k=7 0.293 -> 0.276
         // (no residual) and 0.337 -> 0.313 (accumulate), ups 256->128 1.14 -> 0.37; k=7 with one residual and k=11 are
@@ -850,7 +849,7 @@ static bool pipe_plan(const ConvArgs& a, PipeParams& p, size_t* smem_out) {
     memset(&p, 0, sizeof(p));
     p.Cin = a.Cin; p.kchunks = a.w16_cin_pad / 64; p.cch = a.Cin == 32 ? 32 : 64;
     p.x16in = a.x16in; p.is_bf16 = a.fmt16 == DT_BF16 ? 1 : 0;
-    p.k32 = (a.Cin == 32 && !tune().no_k32) ? 1 : 0;
+    p.k32 = a.Cin == 32 ? 1 : 0;
     const int ph = a.phases;               // 1, or the stride of a transposed conv (columns = ph * Cout)
     const bool tr_ = a.phases > 1;
     p.B = a.B; p.M = a.M; p.Tin = a.Tin; p.Cout = ph * a.Cout;
@@ -868,17 +867,13 @@ static bool pipe_plan(const ConvArgs& a, PipeParams& p, size_t* smem_out) {
         // 12 KB blocks by default; 8 KB when every residual stage holds two boxes (residual + accumulate), where the
         // smaller blocks leave room for one more stage (measured: 0.75 -> 0.60 ms on the 32-channel k=11 layer)
         int xmax = (a.res != nullptr && a.accumulate) ? 8192 : P_XSLOT_MAX;
-        // measured per layer class on the B200 (tools/sweep_pipe.sh, ST2_PIPE_XMAX): 8 KB blocks win by 3-14 % where the 12 KB
+        // measured per layer class on the B200: 8 KB blocks win by 3-14 % where the 12 KB
         // split leaves a short last block per tile -- 64 channels k=7 (0.435 -> 0.398 ms), 128 channels k=3 without residual
         // (0.362 -> 0.312) and k=7 with one residual (0.350 -> 0.338); every 32-channel layer loses 5-14 % with them
         const int nres_ = (a.res != nullptr ? 1 : 0) + (a.accumulate ? 1 : 0);
         if ((a.Cin == 64 && a.ntaps == 7) || (a.Cin == 128 && a.ntaps == 3 && nres_ == 0) || (a.Cin == 128 && a.ntaps == 7 && nres_ == 1))
             xmax = 8192;
-        { const int v = tune().pipe_xmax; if (v >= 2048 && v <= P_XSLOT_MAX) xmax = v; }
-        if (a.x16in) {
-            if (xmax > 8192) xmax = 8192;     // fp16 input: a 12 KB block would be a whole tile for one warp (8 KB: 1-8 % faster on the k=3 layers)
-            { const int v = tune().pipe_xmax16; if (v >= 1024 && v <= P_XSLOT_MAX) xmax = v; }
-        }
+        if (a.x16in && xmax > 8192) xmax = 8192;  // fp16 input: a 12 KB block would be a whole tile for one warp (8 KB: 1-8 % faster on the k=3 layers)
         int nblk = 1;
         for (;; ++nblk) {
             p.xr = (cdiv(p.rows, nblk) + rpp - 1) / rpp * rpp;
@@ -896,7 +891,6 @@ static bool pipe_plan(const ConvArgs& a, PipeParams& p, size_t* smem_out) {
     p.mtiles = cdiv(a.M, P_MT);
     p.num_tiles = a.B * p.mtiles;
     p.nacc = p.bn <= 128 ? 4 : 2;
-    { const int v = tune().pipe_nacc; if (v == 2 || (v == 4 && p.bn <= 128)) p.nacc = v; }
     p.nacc_log2 = p.nacc == 4 ? 2 : 1;
     int cols = 32;
     while (cols < p.nacc * p.bn) cols <<= 1;
@@ -905,10 +899,8 @@ static bool pipe_plan(const ConvArgs& a, PipeParams& p, size_t* smem_out) {
     p.r16 = a.res16 ? 1 : 0;
     p.o16 = (a.accumulate && a.acc_src != nullptr && a.acc16) ? 1 : 0;
     p.eg = (p.cch == 32 && p.nres > 0 && !tr_) ? 3 : 2;
-    // three groups for the non-residual 32-channel layers too (ST2_PIPE_EG3_NORES=1): measured slower, 0.385 -> 0.416 ms at k = 3 --
-    // the 96-register variant costs the transform warps more than the third group gives the epilogue
-    if (p.cch == 32 && p.nres == 0 && !tr_ && tune().pipe_eg3_nores) p.eg = 3;
-    { const int v = tune().pipe_eg; if (v == 2 || (v == 3 && !tr_)) p.eg = v; }
+    // three groups for the non-residual 32-channel layers too were measured slower, 0.385 -> 0.416 ms at k = 3 -- the
+    // 96-register variant costs the transform warps more than the third group gives the epilogue
     // 3 groups need 4 accumulators: a group's previous tile is tcnt-3, so MMA(tcnt-4) -- the previous use of its accumulator
     // -- has completed when it waits; with 2 accumulators the previous use is tile tcnt-2 and the parity wait could pass early
     if (p.nacc < 4) p.eg = 2;
@@ -928,7 +920,7 @@ static bool pipe_plan(const ConvArgs& a, PipeParams& p, size_t* smem_out) {
     // (measured on the 128-channel layers: conv2 with one residual 0.405 -> 0.36 ms (k=7), 0.535 -> 0.507 (k=11); layers without
     // a residual, whose epilogue staging leaves less room for the rings, and the accumulate layers lose, so only nres == 1)
     const bool pair_ok = p.nt == 1 && p.kchunks == 2 && p.bn <= 128 && p.nacc == 4 && p.nres == 1 &&
-                         (int64_t)a.ntaps * p.kchunks * b_stage > 96 * 1024 && !tune().no_pipe_pair;
+                         (int64_t)a.ntaps * p.kchunks * b_stage > 96 * 1024;
     int na = (pair_ok || p.nt > 1) ? 4 : 2;
     int64_t base = na * a_bytes + 2048 + (p.nres ? 0 : (int64_t)(4 * p.eg) * 4096);
     const int64_t w_resident = (int64_t)a.ntaps * p.kchunks * b_stage;
@@ -951,12 +943,9 @@ static bool pipe_plan(const ConvArgs& a, PipeParams& p, size_t* smem_out) {
     left -= rings(nx, nr);
     int nr_goal = p.nres ? (2 * nchunks + 2 > 8 ? 8 : 2 * nchunks + 2) : 0;
     int nx_goal = 10;
-    { const int v = tune().pipe_nxg; if (v >= 3 && v <= 16) nx_goal = v; }
-    { const int v = tune().pipe_nrg; if (p.nres && v >= 2 && v <= 12) nr_goal = v; }
     // resident weights of a 2-chunk layer (128 channels, k = 3: 96 KB) leave little for the rings: two operand buffers and
     // deeper rings measured 0.319 -> 0.264 ms (no residual), 0.356 -> 0.310 (residual), 0.546 -> 0.478 (accumulate)
     int na_goal = (p.resident && p.kchunks >= 2) ? 2 : 4;
-    { const int v = tune().pipe_na; if (v >= 2 && v <= 4) na_goal = v; }
     for (bool grew = true; grew;) {
         grew = false;
         // a third / fourth operand buffer as soon as the rings hold ~32 KB / ~48 KB each (or all they are allowed to)
@@ -971,8 +960,6 @@ static bool pipe_plan(const ConvArgs& a, PipeParams& p, size_t* smem_out) {
     }
     if (!p.resident)
         while (p.wstages < 8 && left >= b_stage) { ++p.wstages; left -= b_stage; }
-    { const int v = tune().pipe_nx; if (v >= 2 && v <= nx) nx = v; }
-    { const int v = tune().pipe_nr; if (p.nres && v >= 1 && v <= nr) nr = v; }
     p.nx = nx; p.nr = nr;
     p.na = na;
     p.pair = (pair_ok && !p.resident && na == 4) ? 1 : 0;
@@ -1066,7 +1053,7 @@ int launch_conv_pipe(const ConvArgs& a, const float* coef, int coef_ld, int act,
     lattr.val.programmaticStreamSerializationAllowed = 1;
     // Only for small problems (a few tiles per CTA, i.e. one-sentence latency: 3.65 -> 3.29 ms at 1 x 3 s): in throughput
     // runs the early CTAs of this kernel sit on SMs the coefficient kernel in front of it needs, +0.8 ms per 64 x 5 s step
-    const bool pdl = !tune().no_pdl && (p.num_tiles <= 16 * num_sms || tune().pdl_always);
+    const bool pdl = p.num_tiles <= 16 * num_sms;
     lcfg.attrs = &lattr; lcfg.numAttrs = pdl ? 1 : 0;
 #define PIPE_LAUNCH(A, BF, X, G)                                                                                         \
     do {                                                                                                                 \

@@ -36,14 +36,6 @@ namespace st2 {
 
 static constexpr int RW_THREADS = 640;                    // 20 warps (ptxas grants 96 registers from 545 threads up)
 static constexpr int RW_X0 = 2;                          // first transform warp
-#ifndef RW_SECTIONS
-// 1: operand buffers are handed over per 128-row section (the MMA of sub-tile s starts when its rows are transformed, the
-// transform of tile m + na starts when the first sub-tiles of tile m are done); 0: per macro tile.  Measured on one box (build
-// variants, tools/gpu_r2h.sh): sections lose on the k >= 7 layers (C = 32 k = 7: 0.284 -> 0.330 ms) -- the extra barrier waits
-// and commits serialise in the single MMA-issuing thread -- and change nothing elsewhere, so the default is per macro tile.
-#define RW_SECTIONS 0
-#endif
-static constexpr int RW_NSEC = 5;                        // 128-row sections of an operand buffer: sub (<= 4) + the halo section
 static constexpr int RW_MAXGRID = 160;                   // statistics buffers are sized for at most this many CTAs
 
 // where the partials of an utterance live in the statistics buffer of a conv_row launch (see flush() and RowStatsDesc)
@@ -193,9 +185,9 @@ conv_row_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
     float* coef_s = bias_s + C;                                                  // [J][2][C] in-kernel AdaIN coefficients (<= 2 KB)
     uint64_t* bars = reinterpret_cast<uint64_t*>(coef_s + (p.cin_part != nullptr ? p.J * 2 * C : 0));
     uint64_t* w_full = bars;                    // [1]
-    uint64_t* a_full = bars + 1;                // [4 buffers][RW_NSEC sections of 128 operand rows]
-    uint64_t* a_empty = a_full + 4 * RW_NSEC;   // [4][RW_NSEC]
-    uint64_t* acc_full = a_empty + 4 * RW_NSEC; // [8]
+    uint64_t* a_full = bars + 1;                // [4 operand buffers]
+    uint64_t* a_empty = a_full + 4;             // [4]
+    uint64_t* acc_full = a_empty + 4;           // [8]
     uint64_t* acc_empty = acc_full + 8;         // [8]
     uint64_t* r_full = acc_empty + 8;           // [nr]
     uint64_t* r_empty = r_full + p.nr;          // [nr]
@@ -218,19 +210,11 @@ conv_row_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
         if (p.nres >= 1) prefetch_tmap(&map_r);
         if (p.nres >= 2) prefetch_tmap(&map_o);
         mbar_init(w_full, 1);
-        // operand buffers are handed over in sections of 128 rows: section s < sub is written by 128 / R blocks and read by
-        // sub-tiles s - 1 and s, the halo section (s == sub) by the remaining blocks and the last sub-tile
-        const int bps = 128 / p.R;
-        for (int i = 0; i < p.na; ++i)
-            for (int sec = 0; sec <= p.sub; ++sec) {
-                if (RW_SECTIONS) {
-                    mbar_init(&a_full[i * RW_NSEC + sec], (uint32_t)(sec < p.sub ? bps : p.nblk - p.sub * bps));
-                    mbar_init(&a_empty[i * RW_NSEC + sec], (sec == 0 || sec == p.sub) ? 1u : 2u);
-                } else {
-                    mbar_init(&a_full[i * RW_NSEC + sec], (uint32_t)p.nblk);
-                    mbar_init(&a_empty[i * RW_NSEC + sec], 1u);
-                }
-            }
+        // operand buffers are handed over per macro tile: filled by its nblk blocks, emptied by the MMA of its last sub-tile
+        for (int i = 0; i < p.na; ++i) {
+            mbar_init(&a_full[i], (uint32_t)p.nblk);
+            mbar_init(&a_empty[i], 1u);
+        }
         for (int i = 0; i < 8; ++i) {
             mbar_init(&acc_full[i], 1);
             mbar_init(&acc_empty[i], (uint32_t)(4 * NCH));   // the warps that drain one accumulator
@@ -344,21 +328,13 @@ conv_row_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
             int b = m_lo / p.mmt, mm = m_lo - b * p.mmt;
             uint32_t buf = 0, buf_par = 0;              // operand buffer of macro tile mc: mc % na, fill parity (mc / na) & 1
             for (int mc = 0; mc < m_n; ++mc) {
-                uint64_t* af = a_full + buf * RW_NSEC;
-                uint64_t* ae = a_empty + buf * RW_NSEC;
                 for (int s = 0; s < p.sub; ++s) {
-                    // every section is waited for exactly once per fill (a parity wait only tells adjacent phases apart), also
-                    // by the sub-tiles past the end of the utterance, which contract nothing but still hand their sections back
-                    if (s == 0) mbar_wait(&af[0], buf_par);
-                    if (RW_SECTIONS) mbar_wait(&af[s + 1], buf_par);          // rows [128 s, 128 s + 128 + span) are transformed
+                    // the buffer is waited for exactly once per fill (a parity wait only tells adjacent phases apart) and handed
+                    // back also when its last sub-tiles lie past the end of the utterance and contract nothing
+                    if (s == 0) mbar_wait(&a_full[buf], buf_par);
                     tc_fence_after();
                     if (mm * sub_rows + s * 128 >= p.M) {
-                        if (RW_SECTIONS) {
-                            umma_commit(&ae[s]);
-                            umma_commit(&ae[s + 1]);
-                        } else if (s == p.sub - 1) {
-                            umma_commit(&ae[0]);
-                        }
+                        if (s == p.sub - 1) umma_commit(&a_empty[buf]);
                         continue;
                     }
                     const uint32_t acc = sc & (uint32_t)(p.nacc - 1);
@@ -397,12 +373,7 @@ conv_row_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                         b_lo += btile >> 4;
                     }
                     umma_commit(&acc_full[acc]);
-                    if (RW_SECTIONS) {
-                        umma_commit(&ae[s]);                 // one of the (at most) two readers of each section is done
-                        umma_commit(&ae[s + 1]);
-                    } else if (s == p.sub - 1) {
-                        umma_commit(&ae[0]);
-                    }
+                    if (s == p.sub - 1) umma_commit(&a_empty[buf]);
                     ++sc;
                 }
                 if (++buf == (uint32_t)p.na) { buf = 0; buf_par ^= 1u; }
@@ -478,8 +449,7 @@ conv_row_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                 const int nvalid = (blk == p.nblk - 1) ? p.tail_rows : p.R;      // rows the TMA box really loaded
                 const int t0 = mm * sub_rows + p.halo_min + r0;                  // time index of operand row r0
                 mbar_wait_warp(&x_full[slot], xpar);
-                const uint32_t sec = RW_SECTIONS ? (uint32_t)r0 >> 7 : 0u;      // 128-row section of the operand buffer
-                mbar_wait_warp(&a_empty[buf * RW_NSEC + sec], (fill & 1u) ^ 1u);
+                mbar_wait_warp(&a_empty[buf], (fill & 1u) ^ 1u);
                 uint32_t xaddr = smem_x_u32 + slot * (uint32_t)p.xslot + (uint32_t)rl * xrow + (uint32_t)c4 * xes;
                 uint32_t abase = smem_a_u32 + buf * (uint32_t)p.a_bytes + (uint32_t)r0 * arow;
                 // whole batches: rows past nvalid read stale slot bytes and land in slack operand rows no MMA reads
@@ -512,7 +482,7 @@ conv_row_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                 fence_proxy_async();
                 __syncwarp();                                        // every lane has read the slot and written its rows
                 if (lane == 0) {
-                    mbar_arrive(&a_full[buf * RW_NSEC + sec]);
+                    mbar_arrive(&a_full[buf]);
                     if (l_mi < m_n) issue_load();                    // refill the slot just consumed (l_i == xi)
                 }
                 if (l_mi < m_n) advance_load();
@@ -668,7 +638,6 @@ int make_map_3d_sw(CUtensorMap* map, int dtype, const void* base, uint64_t d0, u
                    uint64_t stride2_bytes, uint32_t b0, uint32_t b1, int swizzle_bytes);
 
 static int row_num_sms() { return device_num_sms(); }
-static bool row_disabled() { return tune().no_row != 0; }
 
 static bool row_geometry_ok(const ConvArgs& a) {
     if (a.in_stride != 1 || a.mirror || a.res_shift != 0 || a.phases != 1) return false;
@@ -699,7 +668,7 @@ static bool row_plan(const ConvArgs& a, RowParams& p, size_t* smem_out, int* gri
     p.tmem_cols = 256;
     // the bias through the tensor core: 32-channel layers with scale 1 (every conv of a resblock but the last of a stage); the
     // 64-channel layers run 8 epilogue warps and have no shared memory to spare for an 8 KB bias tile
-    p.bias_mma = (nch == 1 && a.bias != nullptr && a.scale == 1.f && !tune().no_row_bias_mma) ? 1 : 0;
+    p.bias_mma = (nch == 1 && a.bias != nullptr && a.scale == 1.f) ? 1 : 0;
     const int ntw = 18 - 4 * nch;
     const int xes = a.x16in ? 2 : 4;
     const int brows = nch == 1 ? 32 : 16;                  // rows per transform batch
@@ -709,7 +678,6 @@ static bool row_plan(const ConvArgs& a, RowParams& p, size_t* smem_out, int* gri
     // 64-channel k = 3 layer) with the largest macro tile that fits (the halo is transformed once per macro tile), then the
     // deepest rings; 2 KB blocks only where nothing else fits
     for (int slot_bytes = 4096; slot_bytes >= 2048 && !ok; slot_bytes >>= 1) {
-        if (tune().row_slot && slot_bytes != tune().row_slot) continue;
         for (int sub = 4; sub >= 1 && !ok; sub >>= 1) {
             if (tune().row_sub && sub != tune().row_sub) continue;
             const int mr = sub * 128 + span;
@@ -722,25 +690,24 @@ static bool row_plan(const ConvArgs& a, RowParams& p, size_t* smem_out, int* gri
             const int xslot = R * C * xes;
             // three operand buffers for single-sub-tile macro tiles when they fit (the MMA of tile m otherwise gates the
             // transform of tile m + 2 after every 128 rows)
-            for (int na = (tune().row_na >= 2 && tune().row_na <= 4 ? tune().row_na : (sub == 1 ? 3 : 2)); na >= 2 && !ok; --na) {
-            if (tune().row_na && na != tune().row_na) continue;
-            const int lw_max = na * nblk < ntw ? na * nblk : ntw;
-            const int64_t fixed = na * a_bytes + (int64_t)a.ntaps * btile + btile + 4096 + (p.bias_mma ? btile + 1024 : 0);
-            const int nr_max = p.nres ? 4 : 0, nr_min = p.nres ? 2 : 0;
-            // as many transform warps as have a ring (at least 10; 7 for the smallest macro tile) with the deepest rings that fit
-            for (int lw = lw_max; lw >= (lw_max < 10 ? lw_max : (sub == 1 ? 7 : 10)) && !ok; --lw) {
-                for (int nr = nr_max; nr >= nr_min && !ok; --nr) {
-                    for (int xd = 3; xd >= 2 && !ok; --xd) {
-                        const int64_t tot = fixed + (int64_t)nr * p.nres * rtile + (int64_t)lw * xd * xslot;
-                        if (tot <= budget) {
-                            p.sub = sub; p.R = R; p.nblk = nblk; p.tail_rows = tail; p.xslot = xslot; p.a_bytes = (int)a_bytes;
-                            p.lw = lw; p.xd = xd; p.nr = nr; p.na = na;
-                            *smem_out = (size_t)tot + 1024;
-                            ok = true;
+            for (int na = sub == 1 ? 3 : 2; na >= 2 && !ok; --na) {
+                const int lw_max = na * nblk < ntw ? na * nblk : ntw;
+                const int64_t fixed = na * a_bytes + (int64_t)a.ntaps * btile + btile + 4096 + (p.bias_mma ? btile + 1024 : 0);
+                const int nr_max = p.nres ? 4 : 0, nr_min = p.nres ? 2 : 0;
+                // as many transform warps as have a ring (at least 10; 7 for the smallest macro tile) with the deepest rings that fit
+                for (int lw = lw_max; lw >= (lw_max < 10 ? lw_max : (sub == 1 ? 7 : 10)) && !ok; --lw) {
+                    for (int nr = nr_max; nr >= nr_min && !ok; --nr) {
+                        for (int xd = 3; xd >= 2 && !ok; --xd) {
+                            const int64_t tot = fixed + (int64_t)nr * p.nres * rtile + (int64_t)lw * xd * xslot;
+                            if (tot <= budget) {
+                                p.sub = sub; p.R = R; p.nblk = nblk; p.tail_rows = tail; p.xslot = xslot; p.a_bytes = (int)a_bytes;
+                                p.lw = lw; p.xd = xd; p.nr = nr; p.na = na;
+                                *smem_out = (size_t)tot + 1024;
+                                ok = true;
+                            }
                         }
                     }
                 }
-            }
             }
         }
     }
@@ -770,7 +737,7 @@ bool conv_row_can_launch(const ConvArgs& a) {
 // tiles spread them over more SMs.  Tune::row_always drops that threshold (geometry and plan still apply), so the decoder's
 // reference fixtures, a few utterances long, can run every 32 / 64-channel resblock conv on this kernel.
 bool conv_row_supported(const ConvArgs& a) {
-    if (row_disabled() || !row_geometry_ok(a)) return false;
+    if (!row_geometry_ok(a)) return false;
     RowParams p;
     size_t smem;
     int grid;

@@ -41,10 +41,6 @@ struct TcParams {
     int stages;
     float scale; int accumulate; int mirror;
     int is_bf16;
-    // halo mode (kchunks == 1): the A tile is fetched ONCE with halo_rows = 128 + (ntaps-1)*|tap_step| rows and
-    // every tap reads it through a UMMA descriptor whose start address is shifted by whole 128-byte rows
-    int halo_rows;               // 0 = off
-    int halo_min;                // smallest time offset of any tap relative to m0
     int epi_gelu;                // y = GELU(acc + bias) as 16-bit values (is_bf16 selects the format), pitch ld_y elements
 };
 
@@ -55,14 +51,12 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     const uint32_t b_stage_bytes = (uint32_t)p.bn * TC_KC * 2;
     uint8_t* smem_a = smem;
-    const size_t a_region = p.halo_rows ? (size_t)256 * 128 : (size_t)p.stages * A_STAGE_BYTES;
-    uint8_t* smem_b = smem + a_region;
+    uint8_t* smem_b = smem + (size_t)p.stages * A_STAGE_BYTES;
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem_b + (size_t)p.stages * b_stage_bytes);
     uint64_t* full_bar = bars;                     // [stages]
     uint64_t* empty_bar = bars + p.stages;         // [stages]
     uint64_t* tmem_full_bar = bars + 2 * p.stages; // [1]
-    uint64_t* a_full_bar = bars + 2 * p.stages + 1; // [1] (halo mode)
-    uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 2 * p.stages + 2);
+    uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 2 * p.stages + 1);
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
@@ -80,7 +74,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
             mbar_init(&empty_bar[s], 1);
         }
         mbar_init(tmem_full_bar, 1);
-        mbar_init(a_full_bar, 1);
         fence_barrier_init();
     }
     if (warp == 1) {
@@ -99,18 +92,13 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         if (lane == 0) {
             int stage = 0;
             uint32_t phase = 0;
-            if (p.halo_rows) {
-                mbar_expect_tx(a_full_bar, (uint32_t)p.halo_rows * 128u);
-                tma_load_3d(smem_a, &map_a, a_full_bar, 0, m0 + p.halo_min, b);
-            }
             for (int it = 0; it < nit; ++it) {
                 const int j = it / p.kchunks;
                 const int kc = it - j * p.kchunks;
                 mbar_wait(&empty_bar[stage], phase ^ 1);
-                mbar_expect_tx(&full_bar[stage], (p.halo_rows ? 0u : A_STAGE_BYTES) + b_stage_bytes);
-                if (!p.halo_rows)
-                    tma_load_3d(smem_a + (size_t)stage * A_STAGE_BYTES, &map_a, &full_bar[stage], kc * TC_KC,
-                                m0 + j * p.tap_step + p.in_off, b);
+                mbar_expect_tx(&full_bar[stage], A_STAGE_BYTES + b_stage_bytes);
+                tma_load_3d(smem_a + (size_t)stage * A_STAGE_BYTES, &map_a, &full_bar[stage], kc * TC_KC,
+                            m0 + j * p.tap_step + p.in_off, b);
                 tma_load_3d(smem_b + (size_t)stage * b_stage_bytes, &map_b, &full_bar[stage], kc * TC_KC, n0,
                             ph + j * p.w_step);
                 if (++stage == p.stages) { stage = 0; phase ^= 1; }
@@ -122,13 +110,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
             const uint32_t idesc = umma_idesc(TC_BM, p.bn, p.is_bf16);
             int stage = 0;
             uint32_t phase = 0;
-            if (p.halo_rows) mbar_wait(a_full_bar, 0);
             for (int it = 0; it < nit; ++it) {
                 mbar_wait(&full_bar[stage], phase);
                 tc_fence_after();
-                const uint64_t adesc = p.halo_rows
-                    ? umma_desc_sw128(smem_u32(smem_a + (size_t)(it * p.tap_step + p.in_off - p.halo_min) * 128))
-                    : umma_desc_sw128(smem_u32(smem_a + (size_t)stage * A_STAGE_BYTES));
+                const uint64_t adesc = umma_desc_sw128(smem_u32(smem_a + (size_t)stage * A_STAGE_BYTES));
                 const uint64_t bdesc = umma_desc_sw128(smem_u32(smem_b + (size_t)stage * b_stage_bytes));
 #pragma unroll
                 for (int k4 = 0; k4 < TC_KC / 16; ++k4)
@@ -483,25 +468,18 @@ int launch_conv_tc(const ConvArgs& a, cudaStream_t st) {
     int cols = 32;
     while (cols < bn) cols <<= 1;
     p.tmem_cols = cols;
-    const bool want_halo = tune().tc_halo != 0;
-    const int span = (a.ntaps - 1) * (a.tap_step < 0 ? -a.tap_step : a.tap_step);
-    if (want_halo && p.kchunks == 1 && TC_BM + span <= 256) {
-        p.halo_rows = TC_BM + span;
-        p.halo_min = a.in_off + (a.tap_step < 0 ? (a.ntaps - 1) * a.tap_step : 0);
-    }
-    const uint32_t stage_bytes = (p.halo_rows ? 0 : A_STAGE_BYTES) + (uint32_t)bn * TC_KC * 2;
-    int stages = (int)((96 * 1024 - (p.halo_rows ? 32 * 1024 : 0)) / stage_bytes);   // <= 96 KB: two CTAs per SM
+    const uint32_t stage_bytes = A_STAGE_BYTES + (uint32_t)bn * TC_KC * 2;
+    int stages = (int)(96 * 1024 / stage_bytes);   // <= 96 KB: two CTAs per SM
     if (stages > 6) stages = 6;
     if (stages < 2) stages = 2;
     p.stages = stages;
-    const size_t smem = (size_t)stages * stage_bytes + (p.halo_rows ? 32 * 1024 : 0) + (2 * stages + 2) * sizeof(uint64_t) +
-                        16 + 1024;
+    const size_t smem = (size_t)stages * stage_bytes + (2 * stages + 2) * sizeof(uint64_t) + 16 + 1024;
 
     CUtensorMap map_a, map_b;
     const int ktaps_total = a.phases > 1 ? a.ntaps * a.phases : a.ntaps;   // weight taps stored
     const uint64_t a_d0 = (uint64_t)(a.ld_x16 < a.w16_cin_pad ? a.ld_x16 : a.w16_cin_pad);
     int e = make_map_3d(&map_a, is_bf16, a.x16, a_d0, (uint64_t)a.Tin, (uint64_t)a.B, (uint64_t)a.ld_x16 * 2,
-                        (uint64_t)a.Tin * a.ld_x16 * 2, TC_KC, p.halo_rows ? (uint32_t)p.halo_rows : (uint32_t)TC_BM);
+                        (uint64_t)a.Tin * a.ld_x16 * 2, TC_KC, (uint32_t)TC_BM);
     if (e != ST2_OK) return e;
     e = make_map_3d(&map_b, is_bf16, a.w16, (uint64_t)a.w16_cin_pad, (uint64_t)a.w16_cout_pad, (uint64_t)ktaps_total,
                     (uint64_t)a.w16_cin_pad * 2, (uint64_t)a.w16_cin_pad * a.w16_cout_pad * 2, TC_KC, (uint32_t)bn);

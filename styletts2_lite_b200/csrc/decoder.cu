@@ -346,7 +346,7 @@ static int forward_impl(st2_decoder* d, const float* asr, const float* f0, const
         Exec::StatRef xu_stats{nullptr, 0, true};
         const bool fuse_u = E.can_fuse(d->ups[i], dtu, Cin, C, u, 1);
         // The stage input xu = ups(x) + x_source is read six times (input and residual of the first iteration of the three
-        // resblocks): stored as fp16 when the ups conv and all six convs run on the TMA pipeline kernel (ST2_NO_XU16=1: fp32)
+        // resblocks): stored as fp16 when the ups conv and all six convs run on the TMA pipeline kernel (fp16_xu = 0: fp32)
         int xu16 = 0;
         if (fuse_u && d->opt_xu16 && E.pipe_ok_ups16(d->ups[i], Cin, C, Tin, Tout, u, pu, shift, dtu)) {
             xu16 = 1;
@@ -372,7 +372,7 @@ static int forward_impl(st2_decoder* d, const float* asr, const float* f0, const
         else E.tap("generator.stage" + is + ".in", xu, C, (int64_t)B * Tout, C);
         float* run = E.allocf((int64_t)B * Tout * C);
         // the partial sum over the resblocks of the stage (written by the first, read + written by the middle ones, read by the
-        // last, which writes the fp32 stage output) is kept in fp16 when all their last convs take it (ST2_NO_SUM16=1: fp32)
+        // last, which writes the fp32 stage output) is kept in fp16 when all their last convs take it (fp16_sum = 0: fp32)
         void* sum16buf = E.alloc((int64_t)B * Tout * C * 2);
         int sum16 = c.n_kernels >= 2 ? 1 : 0;
         for (int j = 0; j < c.n_kernels && sum16; ++j)
@@ -417,33 +417,12 @@ static int forward_impl(st2_decoder* d, const float* asr, const float* f0, const
 
 // ---- process-wide tuning switches (common.cuh)
 namespace {
-struct TuneField { const char* name; const char* env; int Tune::*field; bool flag; };
+struct TuneField { const char* name; int Tune::*field; };
 const TuneField kTuneFields[] = {
-    {"no_pdl", "ST2_NO_PDL", &Tune::no_pdl, true}, {"pdl_always", "ST2_PDL_ALWAYS", &Tune::pdl_always, true},
-    {"no_k32", "ST2_NO_K32", &Tune::no_k32, true}, {"no_xstage", "ST2_NO_XSTAGE", &Tune::no_xstage, true},
-    {"no_fused", "ST2_NO_FUSED", &Tune::no_fused, true}, {"no_pipe", "ST2_NO_PIPE", &Tune::no_pipe, true},
-    {"no_pipe_ups", "ST2_NO_PIPE_UPS", &Tune::no_pipe_ups, true}, {"no_pipe_nt", "ST2_NO_PIPE_NT", &Tune::no_pipe_nt, true},
-    {"no_pipe_pair", "ST2_NO_PIPE_PAIR", &Tune::no_pipe_pair, true}, {"no_row", "ST2_NO_ROW", &Tune::no_row, true},
-    {"pipe_xmax", "ST2_PIPE_XMAX", &Tune::pipe_xmax, false}, {"pipe_xmax16", "ST2_PIPE_XMAX16", &Tune::pipe_xmax16, false},
-    {"pipe_nacc", "ST2_PIPE_NACC", &Tune::pipe_nacc, false}, {"pipe_eg3_nores", "ST2_PIPE_EG3_NORES", &Tune::pipe_eg3_nores, true},
-    {"pipe_eg", "ST2_PIPE_EG", &Tune::pipe_eg, false}, {"pipe_nxg", "ST2_PIPE_NXG", &Tune::pipe_nxg, false},
-    {"pipe_nrg", "ST2_PIPE_NRG", &Tune::pipe_nrg, false}, {"pipe_na", "ST2_PIPE_NA", &Tune::pipe_na, false},
-    {"pipe_nx", "ST2_PIPE_NX", &Tune::pipe_nx, false}, {"pipe_nr", "ST2_PIPE_NR", &Tune::pipe_nr, false},
-    {"verbose", "ST2_PIPE_VERBOSE", &Tune::verbose, true}, {"tc_halo", "ST2_TC_HALO", &Tune::tc_halo, false},
-    {"no_row_bias_mma", "ST2_NO_ROW_BIAS_MMA", &Tune::no_row_bias_mma, true}, {"no_row_inline_coef", "ST2_NO_ROW_INLINE_COEF", &Tune::no_row_inline_coef, true},
-    {"lstm_bt", "ST2_LSTM_BT", &Tune::lstm_bt, false}, {"no_xt16", "ST2_NO_XT16", &Tune::no_xt16, true},
-    {"no_run16", "ST2_NO_RUN16", &Tune::no_run16, true}, {"no_xu16", "ST2_NO_XU16", &Tune::no_xu16, true},
-    {"no_sum16", "ST2_NO_SUM16", &Tune::no_sum16, true}, {"no_src16", "ST2_NO_SRC16", &Tune::no_src16, true},
-    {"no_out16", "ST2_NO_OUT16", &Tune::no_out16, true}, {"row_sub", "ST2_ROW_SUB", &Tune::row_sub, false},
-    {"row_slot", "ST2_ROW_SLOT", &Tune::row_slot, false}, {"row_na", "ST2_ROW_NA", &Tune::row_na, false},
-    {"row_always", "ST2_ROW_ALWAYS", &Tune::row_always, true}};
+    {"no_pipe", &Tune::no_pipe}, {"row_always", &Tune::row_always}, {"row_sub", &Tune::row_sub},
+    {"no_row_inline_coef", &Tune::no_row_inline_coef}, {"verbose", &Tune::verbose}};
 Tune& tune_storage() {
-    static Tune t = [] {
-        Tune v;
-        for (const TuneField& f : kTuneFields)
-            if (const char* e = getenv(f.env)) v.*(f.field) = f.flag ? 1 : atoi(e);    // the only getenv calls of the library
-        return v;
-    }();
+    static Tune t;
     return t;
 }
 }  // namespace
@@ -482,7 +461,6 @@ static int create_handle(const st2_config* cfg, st2_decoder** out) {
     st2_decoder* d = new (std::nothrow) st2_decoder();
     ST2_REQUIRE(d != nullptr, "create: out of memory");
     d->cfg = *cfg;
-    d->init_options();
     int dev = 0;
     cudaDeviceProp prop;
     if (cudaGetDevice(&dev) == cudaSuccess && cudaGetDeviceProperties(&prop, dev) == cudaSuccess)

@@ -251,7 +251,7 @@ int launch_lstm_bidir(const float* G, const float* whh, const float* bhh, float*
         mc4 = n;
         if (tune().verbose) fprintf(stderr, "lstm: %d co-resident clusters of 8 CTAs (BT=4 configuration)\n", n);
     }
-    const bool bt4 = tune().lstm_bt == 4 || (tune().lstm_bt != 8 && cdiv(B, 4) * 2 <= mc4);
+    const bool bt4 = cdiv(B, 4) * 2 <= mc4;
     return bt4 ? launch_lstm_v2<4>(G, whh, bhh, y, B, T, lengths, st) : launch_lstm_v2<8>(G, whh, bhh, y, B, T, lengths, st);
 }
 

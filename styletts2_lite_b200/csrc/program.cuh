@@ -79,15 +79,9 @@ struct st2_decoder {
     const uint64_t* seed_dev = nullptr;     // optional device-resident Philox seed (st2_decoder_set_seed_buffer)
     bool tc_ok = false;
     int fp16_storage = 1;                   // st2_decoder_set_option("fp16_storage"): stage-private tensors of the 16-bit paths in fp16
-    // ... and each of the four kinds alone ("fp16_xt", "fp16_run", "fp16_xu", "fp16_sum"; DESIGN.md section 3).  Defaults come
-    // from the process-wide switches once, at create time.
+    // ... and each of the four kinds alone ("fp16_xt", "fp16_run", "fp16_xu", "fp16_sum"; DESIGN.md section 3)
     int opt_xt16 = 1, opt_run16 = 1, opt_xu16 = 1, opt_sum16 = 1;
     int opt_src16 = 1, opt_out16 = 1;       // "fp16_src": noise_convs output (input of noise_res); "fp16_out": last stage's output
-    void init_options() {
-        const st2::Tune& t = st2::tune();
-        opt_xt16 = !t.no_xt16; opt_run16 = !t.no_run16; opt_xu16 = !t.no_xu16; opt_sum16 = !t.no_sum16;
-        opt_src16 = !t.no_src16; opt_out16 = !t.no_out16;
-    }
 
     ResBlk1dW encode, decode[4];
     float *f0_w = nullptr, *f0_b = nullptr, *n_w = nullptr, *n_b = nullptr;
@@ -547,7 +541,7 @@ struct Exec {
         coef_ld = Cpad;
     }
     bool can_fuse(const ConvW& w, int dt, int ld_x, int ld_y, int stride, int dilation) {
-        if (!use_tc(w, dt) || tune().no_fused) return false;
+        if (!use_tc(w, dt)) return false;
         ConvArgs a;
         memset(&a, 0, sizeof(a));
         a.in_stride = 1; a.w16 = w.w16[dt]; a.w16_cin_pad = w.cin_pad; a.w16_cout_pad = w.cout_pad;

@@ -54,6 +54,14 @@ def test_create_validates_config_without_gpu(lib):
     assert lib.st2_decoder_create(C.byref(cc), C.byref(h)) == -1
 
 
+def test_set_tuning_accepts_only_the_test_hooks(lib):
+    for name in (b"no_pipe", b"row_always", b"row_sub", b"no_row_inline_coef", b"verbose"):
+        assert lib.st2_set_tuning(name, 0) == 0, name          # 0 is each hook's default: no state changes
+    for name in (b"pipe_xmax", b"no_row", b"tc_halo", b"no_xt16", b"lstm_bt"):
+        assert lib.st2_set_tuning(name, 0) == -1, name
+        assert b"unknown switch" in lib.st2_last_error()
+
+
 @pytest.mark.parametrize("variant", ["hifigan", "istftnet", "vocos"])
 def test_state_dict_schema_matches_reference(variant):
     schema = json.load(open(os.path.join(ROOT, "tests", "golden", "state_dict_schema.json")))[variant]
