@@ -300,6 +300,21 @@ ST2_API int st2_adain_conv1d_fused(const float* x, const float* h, const float* 
                            int32_t k, int32_t padding, int32_t dilation, float scale, int32_t accumulate,
                            int32_t precision, void* stream);
 
+/* st2_adain_conv1d_fused with the fp16 storage types of the decoder's resblocks (Modules/hifigan.py:65-74, :338-342): x is
+ * stored as fp16 when x16, res when res16, y is written as fp16 and widened when y16.  old [B,T,Cout] (may be NULL, needs
+ * accumulate) is a separate accumulate source replacing the old values in y, stored as fp16 when old16; with old_in_y (needs
+ * old16 and y16) it is first stored into the fp16 y buffer and the conv accumulates in place, as the middle resblock of a
+ * stage updates the fp16 stage sum.  All pointers are fp32 channels-last tensors; the conversions happen in scratch.
+ *   y = (conv1d(act(AdaIN(x; h)), w) + bias + res + old) * scale
+ * Any 16-bit flag needs a geometry the TMA pipeline kernel runs; otherwise ST2_ERR_INVALID. */
+ST2_API int64_t st2_adain_conv1d_fused_ex_scratch_bytes(int32_t B, int32_t T, int32_t Cin, int32_t Cout, int32_t k);
+ST2_API int st2_adain_conv1d_fused_ex(const float* x, const float* h, const float* alpha, int32_t act, float slope,
+                              const float* w, const float* bias, const float* res, const float* old, float* y,
+                              const float* h_next, float* coef_next, void* scratch, int32_t B, int32_t T, int32_t Cin,
+                              int32_t Cout, int32_t k, int32_t padding, int32_t dilation, float scale, int32_t accumulate,
+                              int32_t x16, int32_t res16, int32_t old16, int32_t y16, int32_t old_in_y, int32_t precision,
+                              void* stream);
+
 /* The same half-step (Snake, C = Cin = Cout in {32, 64}) on the row-per-thread kernel with the storage types of the 16-bit
  * decoder paths: res / old (the running tensor and the partial stage sum of Modules/hifigan.py:65-74, :338-342) are stored as
  * fp16 and added by the tensor core; x is stored as fp16 when x16, y is written as fp16 when y16.  All pointers are fp32
@@ -335,6 +350,17 @@ ST2_API int st2_act_conv_transpose1d_fused(const float* x, const float* alpha, i
                                    float* coef_next, void* scratch, int32_t B, int32_t Tin, int32_t Cin, int32_t Cout,
                                    int32_t k, int32_t stride, int32_t padding, int32_t output_padding,
                                    int32_t precision, void* stream);
+
+/* st2_act_conv_transpose1d_fused with the fp16 output of the decoder's upsampling step: with y16, y is written as fp16 (the
+ * stage input the resblocks read) and widened into the fp32 y; that needs a geometry the TMA pipeline kernel runs, otherwise
+ * ST2_ERR_INVALID.  output_padding < stride. */
+ST2_API int64_t st2_act_conv_transpose1d_fused_ex_scratch_bytes(int32_t B, int32_t Tin, int32_t Cin, int32_t Cout, int32_t k,
+                                                        int32_t stride);
+ST2_API int st2_act_conv_transpose1d_fused_ex(const float* x, const float* alpha, int32_t act, float slope, const float* w,
+                                      const float* bias, const float* res, float* y, const float* h_next,
+                                      float* coef_next, void* scratch, int32_t B, int32_t Tin, int32_t Cin, int32_t Cout,
+                                      int32_t k, int32_t stride, int32_t padding, int32_t output_padding, int32_t y16,
+                                      int32_t precision, void* stream);
 
 #ifdef __cplusplus
 }

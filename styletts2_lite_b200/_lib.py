@@ -108,6 +108,9 @@ SIGNATURES = {
     "st2_postprocess_scratch_bytes": (_L, [_I]),
     "st2_postprocess_max_samples": (_L, [_I, _I, _I, _I]),
     "st2_postprocess": (C.c_int, [_P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
+    "st2_adain_conv1d_fused_ex_scratch_bytes": (_L, [_I, _I, _I, _I, _I]),
+    "st2_adain_conv1d_fused_ex": (C.c_int, [_P, _P, _P, _I, C.c_float, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I,
+                                            _I, C.c_float, _I, _I, _I, _I, _I, _I, _I, _P]),
     "st2_adain_conv1d_row_scratch_bytes": (_L, [_I, _I, _I, _I]),
     "st2_adain_conv1d_row": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, C.c_float, _I, _I, _I,
                                        _P]),
@@ -117,6 +120,9 @@ SIGNATURES = {
     "st2_act_conv_transpose1d_fused_scratch_bytes": (_L, [_I, _I, _I, _I, _I, _I]),
     "st2_act_conv_transpose1d_fused": (C.c_int, [_P, _P, _I, C.c_float, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I,
                                                  _I, _P]),
+    "st2_act_conv_transpose1d_fused_ex_scratch_bytes": (_L, [_I, _I, _I, _I, _I, _I]),
+    "st2_act_conv_transpose1d_fused_ex": (C.c_int, [_P, _P, _I, C.c_float, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I,
+                                                    _I, _I, _I, _P]),
     "st2_conv1d": (C.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
 }
 

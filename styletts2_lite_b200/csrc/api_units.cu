@@ -208,6 +208,88 @@ int st2_adain_conv1d_fused(const float* x, const float* h, const float* alpha, i
     return e;
 }
 
+// st2_adain_conv1d_fused with the fp16 storage types of the decoder's resblocks (program.cuh resblock1): x, res, old are given
+// as fp32 tensors and stored as fp16 first when their flag says so; y is written as fp16 and widened when y16.  A separate
+// accumulate source `old` (fp32 or fp16) replaces the old values in y; with old_in_y it is first stored into the fp16 y buffer
+// and the conv accumulates in place, as the middle resblock of a stage updates the fp16 stage sum.
+static int64_t fused_ex_offsets(int B, int T, int Cin, int Cout, int k, int64_t off[11]) {
+    int64_t o = fused_unit_offsets(B, T, Cin, Cout, k, off);
+    off[6] = o; o += align256((int64_t)B * T * Cin * 2);                         // x as fp16
+    off[7] = o; o += align256((int64_t)B * T * Cout * 2);                        // res as fp16
+    off[8] = o; o += align256((int64_t)B * T * Cout * 2);                        // old as fp16
+    off[9] = o; o += align256((int64_t)B * T * Cout * 2);                        // y as fp16
+    off[10] = o;
+    return o;
+}
+
+int64_t st2_adain_conv1d_fused_ex_scratch_bytes(int32_t B, int32_t T, int32_t Cin, int32_t Cout, int32_t k) {
+    if (B <= 0 || T <= 0 || Cin <= 0 || Cout <= 0 || k <= 0) return ST2_ERR_INVALID;
+    int64_t off[11];
+    return fused_ex_offsets(B, T, Cin, Cout, k, off);
+}
+
+int st2_adain_conv1d_fused_ex(const float* x, const float* h, const float* alpha, int32_t act, float slope, const float* w,
+                              const float* bias, const float* res, const float* old, float* y, const float* h_next,
+                              float* coef_next, void* scratch, int32_t B, int32_t T, int32_t Cin, int32_t Cout, int32_t k,
+                              int32_t padding, int32_t dilation, float scale, int32_t accumulate, int32_t x16, int32_t res16,
+                              int32_t old16, int32_t y16, int32_t old_in_y, int32_t precision, void* stream) {
+    ST2_REQUIRE(x && w && y && scratch && B > 0 && T > 0 && Cin > 0 && Cout > 0 && k > 0 && dilation > 0,
+                "adain_conv1d_fused_ex: bad argument");
+    ST2_REQUIRE(precision == ST2_PREC_BF16 || precision == ST2_PREC_FP16, "adain_conv1d_fused_ex: 16-bit precisions only");
+    ST2_REQUIRE(2 * padding == dilation * (k - 1), "adain_conv1d_fused_ex: length-preserving convolutions only");
+    ST2_REQUIRE((h_next == nullptr) == (coef_next == nullptr), "adain_conv1d_fused_ex: h_next and coef_next go together");
+    ST2_REQUIRE(!res16 || res != nullptr, "adain_conv1d_fused_ex: res16 needs a residual");
+    ST2_REQUIRE(old == nullptr || accumulate, "adain_conv1d_fused_ex: a separate accumulate source needs accumulate");
+    ST2_REQUIRE(!old16 || old != nullptr, "adain_conv1d_fused_ex: old16 needs old values");
+    ST2_REQUIRE(!old_in_y || (old16 && y16), "adain_conv1d_fused_ex: old_in_y accumulates in place on an fp16 y (old16, y16)");
+    cudaStream_t st = (cudaStream_t)stream;
+    int64_t off[11];
+    fused_ex_offsets(B, T, Cin, Cout, k, off);
+    char* base = (char*)scratch;
+    float* wp = (float*)(base + off[0]);
+    void* w16 = base + off[1];
+    void* xstats = base + off[2];
+    float* coef = (float*)(base + off[3]);
+    void* parts = base + off[4];
+    void* x16b = base + off[6];
+    void* r16b = base + off[7];
+    void* o16b = base + off[8];
+    void* y16b = base + off[9];
+    const int dt = precision == ST2_PREC_BF16 ? DT_BF16 : DT_F16;
+    const int cin_pad = (Cin + 63) / 64 * 64, cout_pad = (Cout + 31) / 32 * 32;
+    const int64_t n_in = (int64_t)B * T * Cin, n_out = (int64_t)B * T * Cout;
+    int e = launch_fold_pack(nullptr, w, wp, Cout, Cin, k, 0, st);
+    if (e == ST2_OK) e = launch_pack_w16(wp, w16, k, Cin, Cout, cin_pad, cout_pad, dt, st);
+    if (e == ST2_OK && h != nullptr) e = launch_in_stats(x, Cin, B, T, Cin, xstats, st);
+    if (e == ST2_OK) e = launch_adain_coef(xstats, h, 2 * Cin, 0, coef, B, T, Cin, Cin, st);
+    if (e == ST2_OK && x16) e = launch_cast16(x, x16b, n_in, DT_F16, st);
+    if (e == ST2_OK && res16) e = launch_cast16(res, r16b, n_out, DT_F16, st);
+    if (e == ST2_OK && old16) e = launch_cast16(old, old_in_y ? y16b : o16b, n_out, DT_F16, st);
+    if (e != ST2_OK) return e;
+    ConvArgs a;
+    memset(&a, 0, sizeof(a));
+    a.B = B; a.Cin = Cin; a.Cout = Cout; a.Tin = T; a.Tout = T; a.M = T;
+    a.x = x16 ? (const float*)x16b : x; a.ld_x = Cin; a.x16in = x16 ? 1 : 0;
+    a.w = wp; a.w16 = w16; a.w16_cin_pad = cin_pad; a.w16_cout_pad = cout_pad; a.fmt16 = dt;
+    a.bias = bias; a.res = res16 ? (const float*)r16b : res; a.ld_res = Cout; a.res16 = res16 ? 1 : 0;
+    a.y = y16 ? (float*)y16b : y; a.ld_y = Cout; a.y16out = y16 ? 1 : 0;
+    a.ntaps = k; a.tap_step = dilation; a.in_off = -padding; a.in_stride = 1;
+    a.phases = 1; a.w_step = 1; a.out_stride = 1; a.out_pad = 0;
+    a.scale = scale; a.accumulate = accumulate ? 1 : 0;
+    if (old != nullptr) {
+        a.acc_src = old16 ? (old_in_y ? y16b : o16b) : (const void*)old;
+        a.acc16 = old16 ? 1 : 0;
+    }
+    ST2_REQUIRE(conv_fused_supported(a), "adain_conv1d_fused_ex: geometry not supported by the fused kernels");
+    ST2_REQUIRE(!(x16 || res16 || old16 || y16) || conv_pipe_supported(a),
+                "adain_conv1d_fused_ex: these fp16 storage types need the TMA pipeline kernel, which cannot run this geometry");
+    e = launch_conv_fused(a, coef, Cin, act, slope, alpha, h_next ? parts : nullptr, st);
+    if (e == ST2_OK && y16) e = launch_half_to_float(y16b, y, n_out, st);
+    if (e == ST2_OK && h_next != nullptr)
+        e = launch_adain_coef_f2(parts, fused_stats_parts(a), h_next, 2 * Cout, 0, coef_next, B, T, Cout, Cout, st);
+    return e;
+}
+
 // The same half-step on the row-per-thread kernel (conv_row.cu) with the storage types of the 16-bit decoder paths: x, res
 // and old are given as fp32 tensors and are stored as fp16 first when the x16 flag says so / always (res, old); y is written as fp16
 // and widened when y16.  C = Cin = Cout in {32, 64}, Snake only.
@@ -448,6 +530,63 @@ int st2_act_conv_transpose1d_fused(const float* x, const float* alpha, int32_t a
     e = launch_conv_fused(a, coef, Cin, act, slope, alpha, h_next ? parts : nullptr, st);
     if (e != ST2_OK) return e;
     if (h_next != nullptr) e = launch_adain_coef_f2(parts, fused_stats_parts(a), h_next, 2 * Cout, 0, coef_next, B, a.Tout, Cout, Cout, st);
+    return e;
+}
+
+// st2_act_conv_transpose1d_fused with the fp16 output of the decoder's upsampling step (decoder.cu, fp16_xu): with y16 the
+// stage input is written as fp16 and widened into y.
+int64_t st2_act_conv_transpose1d_fused_ex_scratch_bytes(int32_t B, int32_t Tin, int32_t Cin, int32_t Cout, int32_t k,
+                                                        int32_t stride) {
+    if (B <= 0 || Tin <= 0 || Cin <= 0 || Cout <= 0 || k <= 0 || stride <= 0) return ST2_ERR_INVALID;
+    int64_t off[5];
+    const int64_t Tmax = (int64_t)Tin * stride + k;               // >= Tout for any padding >= 0, output_padding < stride
+    return fused_t_offsets(B, Tin, Cin, Cout, k, stride, off) + align256((int64_t)B * Tmax * Cout * 2);   // + y as fp16
+}
+
+int st2_act_conv_transpose1d_fused_ex(const float* x, const float* alpha, int32_t act, float slope, const float* w,
+                                      const float* bias, const float* res, float* y, const float* h_next, float* coef_next,
+                                      void* scratch, int32_t B, int32_t Tin, int32_t Cin, int32_t Cout, int32_t k,
+                                      int32_t stride, int32_t padding, int32_t output_padding, int32_t y16, int32_t precision,
+                                      void* stream) {
+    ST2_REQUIRE(x && w && y && scratch && B > 0 && Tin > 0 && Cin > 0 && Cout > 0 && k > 0 && stride > 0 && padding >= 0 &&
+                    output_padding >= 0 && output_padding < stride,
+                "act_conv_transpose1d_fused_ex: bad argument");
+    ST2_REQUIRE(precision == ST2_PREC_BF16 || precision == ST2_PREC_FP16, "act_conv_transpose1d_fused_ex: 16-bit precisions only");
+    ST2_REQUIRE(k % stride == 0, "act_conv_transpose1d_fused_ex: k must be a multiple of stride");
+    ST2_REQUIRE((h_next == nullptr) == (coef_next == nullptr), "act_conv_transpose1d_fused_ex: h_next and coef_next go together");
+    cudaStream_t st = (cudaStream_t)stream;
+    int64_t off[5];
+    fused_t_offsets(B, Tin, Cin, Cout, k, stride, off);
+    char* base = (char*)scratch;
+    float* wp = (float*)(base + off[0]);
+    void* w16 = base + off[1];
+    float* coef = (float*)(base + off[2]);
+    void* parts = base + off[3];
+    void* y16b = base + off[4];
+    const int dt = precision == ST2_PREC_BF16 ? DT_BF16 : DT_F16;
+    const int cin_pad = (Cin + 63) / 64 * 64, cout_pad = (Cout + 31) / 32 * 32;
+    int e = launch_fold_pack(nullptr, w, wp, Cin, Cout, k, 1, st);
+    if (e == ST2_OK) e = launch_pack_w16(wp, w16, k, Cin, Cout, cin_pad, cout_pad, dt, st);
+    if (e == ST2_OK) e = launch_adain_coef(nullptr, nullptr, 0, 0, coef, B, Tin, Cin, Cin, st);
+    if (e != ST2_OK) return e;
+    ConvArgs a;
+    memset(&a, 0, sizeof(a));
+    a.B = B; a.Cin = Cin; a.Cout = Cout; a.Tin = Tin;
+    a.Tout = (Tin - 1) * stride - 2 * padding + (k - 1) + output_padding + 1;
+    ST2_REQUIRE(a.Tout > 0, "act_conv_transpose1d_fused_ex: empty output");
+    a.x = x; a.ld_x = Cin; a.w = wp; a.w16 = w16; a.w16_cin_pad = cin_pad; a.w16_cout_pad = cout_pad; a.fmt16 = dt;
+    a.bias = bias; a.res = res; a.ld_res = Cout; a.y = y16 ? (float*)y16b : y; a.ld_y = Cout; a.y16out = y16 ? 1 : 0;
+    a.ntaps = k / stride; a.tap_step = -1; a.in_off = 0; a.in_stride = 1;
+    a.phases = stride; a.w_step = stride; a.out_stride = stride; a.out_pad = padding;
+    a.M = (a.Tout - 1 + padding) / stride + 1;
+    a.scale = 1.f;
+    ST2_REQUIRE(conv_fused_supported(a), "act_conv_transpose1d_fused_ex: geometry not supported by the fused kernels");
+    ST2_REQUIRE(!y16 || conv_pipe_supported(a),
+                "act_conv_transpose1d_fused_ex: an fp16 output needs the TMA pipeline kernel, which cannot run this geometry");
+    e = launch_conv_fused(a, coef, Cin, act, slope, alpha, h_next ? parts : nullptr, st);
+    if (e == ST2_OK && y16) e = launch_half_to_float(y16b, y, (int64_t)B * a.Tout * Cout, st);
+    if (e == ST2_OK && h_next != nullptr)
+        e = launch_adain_coef_f2(parts, fused_stats_parts(a), h_next, 2 * Cout, 0, coef_next, B, a.Tout, Cout, Cout, st);
     return e;
 }
 

@@ -758,6 +758,11 @@ int launch_conv_fused(const ConvArgs& a, const float* coef, int coef_ld, int act
     }
     int grid = num_sms;
     if (grid > p.num_tiles) grid = p.num_tiles;
+    if (tune().verbose)
+        fprintf(stderr, "conv_fused: Cin=%d Cout=%d taps=%d step=%d phases=%d mtiles=%d ntile_n=%d bn=%d tiles=%d grid=%d resident=%d "
+                "stages=%d xstage=%d res=%d acc=%d x16=%d y16=%d smem=%zu\n",
+                a.Cin, a.Cout, p.ntaps, p.tap_step, p.phases, p.mtiles, p.ntile_n, p.bn, p.num_tiles, grid, p.resident, p.stages,
+                p.xstage, a.res != nullptr ? 1 : 0, p.accumulate, p.x16in, p.y16out, smem);
     switch (act) {
         case ACT_NONE: conv_fused_kernel<ACT_NONE><<<grid, F_THREADS, smem, st>>>(map_b, map_x, p); break;
         case ACT_LRELU: conv_fused_kernel<ACT_LRELU><<<grid, F_THREADS, smem, st>>>(map_b, map_x, p); break;

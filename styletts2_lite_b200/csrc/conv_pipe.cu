@@ -1039,10 +1039,6 @@ int launch_conv_pipe(const ConvArgs& a, const float* coef, int coef_ld, int act,
     }
     int grid = num_sms;
     if (grid > p.num_tiles) grid = p.num_tiles;
-    if (tune().verbose)
-        fprintf(stderr, "conv_pipe: Cin=%d Cout=%d taps=%d step=%d rows=%d nblk=%d tail=%d xr=%d resident=%d wstages=%d na=%d nacc=%d lw=%d nx=%d nr=%d nres=%d smem=%zu tiles=%d\n",
-                p.Cin, p.Cout, p.ntaps, p.tap_step, p.rows, p.nblk, p.tail_rows, p.xr, p.resident, p.wstages, p.na, p.nacc, p.lw, p.nx, p.nr, p.nres, smem,
-                p.num_tiles);
     ST2_REQUIRE(act != ACT_SNAKE || alpha != nullptr, "conv_pipe: snake needs alpha");
     ST2_REQUIRE(!a.x16in || act == ACT_SNAKE, "conv_pipe: 16-bit input is only built for the Snake transform");
     if (act != ACT_SNAKE) p.eg = 2;                          // the 3-group variant is only built for Snake
@@ -1055,6 +1051,15 @@ int launch_conv_pipe(const ConvArgs& a, const float* coef, int coef_ld, int act,
     // runs the early CTAs of this kernel sit on SMs the coefficient kernel in front of it needs, +0.8 ms per 64 x 5 s step
     const bool pdl = p.num_tiles <= 16 * num_sms;
     lcfg.attrs = &lattr; lcfg.numAttrs = pdl ? 1 : 0;
+    // Cout counts the columns of one accumulator row (phases * Cout for a transposed conv); mtiles * B = tiles, walked
+    // tile = blockIdx.x + i * grid
+    if (tune().verbose)
+        fprintf(stderr, "conv_pipe: Cin=%d Cout=%d phases=%d taps=%d step=%d rows=%d nblk=%d tail=%d xr=%d resident=%d wstages=%d na=%d "
+                "nacc=%d lw=%d nx=%d nr=%d nres=%d smem=%zu mtiles=%d tiles=%d grid=%d pair=%d eg=%d nt=%d bn=%d x16=%d r16=%d o16=%d "
+                "y16=%d pdl=%d\n",
+                p.Cin, p.Cout, p.ostride, p.ntaps, p.tap_step, p.rows, p.nblk, p.tail_rows, p.xr, p.resident, p.wstages, p.na, p.nacc,
+                p.lw, p.nx, p.nr, p.nres, smem, p.mtiles, p.num_tiles, grid, p.pair, p.eg, p.nt, p.bn, p.x16in, p.r16, p.o16,
+                p.y16out, pdl ? 1 : 0);
 #define PIPE_LAUNCH(A, BF, X, G)                                                                                         \
     do {                                                                                                                 \
         lcfg.blockDim = dim3((P_W_EPI0 + 4 * G) * 32);                                                                   \

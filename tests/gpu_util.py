@@ -211,3 +211,56 @@ def act_conv_transpose1d_fused(x_btc, alpha, act, w, bias, res_btc, h_next, stri
                                                   _lib.PREC[precision], stream()), "act_conv_transpose1d_fused")
     torch.cuda.synchronize()
     return y.cpu().numpy(), (None if cn is None else cn.cpu().numpy())
+
+
+def adain_conv1d_fused_ex(x_btc, h, alpha, act, w, bias, res_btc, old_btc, y_old_btc, h_next, padding, dilation, scale=1.0,
+                          slope=0.0, precision="bf16", x16=False, res16=False, old16=False, y16=False, old_in_y=False):
+    """st2_adain_conv1d_fused_ex: the fused half-step with the decoder's fp16 storage types.  old_btc is the separate accumulate
+    source (stored as fp16 when old16; with old_in_y it is first stored into the fp16 y and the conv accumulates in place);
+    y_old_btc the old values of y for the plain accumulate.  Returns (y [B,T,Cout], coef_next [B,2,Cout] or None)."""
+    lib = _lib.load()
+    B, T, Cin = x_btc.shape
+    Cout, _, k = w.shape
+    xd, wd = to_dev(x_btc), to_dev(w)
+    hd = None if h is None else to_dev(h)
+    ad = None if alpha is None else to_dev(alpha.reshape(-1))
+    bd = None if bias is None else to_dev(bias)
+    rd = None if res_btc is None else to_dev(res_btc)
+    od = None if old_btc is None else to_dev(old_btc)
+    hn = None if h_next is None else to_dev(h_next)
+    cn = None if h_next is None else torch.full((B, 2, Cout), float("nan"), device=dev())
+    y = torch.full((B, T, Cout), float("nan"), device=dev()) if y_old_btc is None else to_dev(y_old_btc)
+    accumulate = old_btc is not None or y_old_btc is not None
+    nbytes = _lib.check(lib.st2_adain_conv1d_fused_ex_scratch_bytes(B, T, Cin, Cout, k), "fused_ex_scratch_bytes")
+    scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev())
+    _lib.check(lib.st2_adain_conv1d_fused_ex(_lib.ptr(xd), _lib.ptr(hd), _lib.ptr(ad), _lib.ACT[act], C.c_float(slope),
+                                             _lib.ptr(wd), _lib.ptr(bd), _lib.ptr(rd), _lib.ptr(od), _lib.ptr(y), _lib.ptr(hn),
+                                             _lib.ptr(cn), _lib.ptr(scratch), B, T, Cin, Cout, k, padding, dilation,
+                                             C.c_float(scale), int(accumulate), int(x16), int(res16), int(old16), int(y16),
+                                             int(old_in_y), _lib.PREC[precision], stream()), "adain_conv1d_fused_ex")
+    torch.cuda.synchronize()
+    return y.cpu().numpy(), (None if cn is None else cn.cpu().numpy())
+
+
+def act_conv_transpose1d_fused_ex(x_btc, alpha, act, w, bias, res_btc, h_next, stride, padding, output_padding, slope=0.0,
+                                  precision="bf16", y16=False):
+    """st2_act_conv_transpose1d_fused_ex: the upsampling step, y written as fp16 (and widened) when y16."""
+    lib = _lib.load()
+    B, T, Cin = x_btc.shape
+    _, Cout, k = w.shape
+    Tout = (T - 1) * stride - 2 * padding + (k - 1) + output_padding + 1
+    xd, wd = to_dev(x_btc), to_dev(w)
+    ad = None if alpha is None else to_dev(alpha.reshape(-1))
+    bd = None if bias is None else to_dev(bias)
+    rd = None if res_btc is None else to_dev(res_btc)
+    hn = None if h_next is None else to_dev(h_next)
+    cn = None if h_next is None else torch.full((B, 2, Cout), float("nan"), device=dev())
+    y = torch.full((B, Tout, Cout), float("nan"), device=dev())
+    nbytes = _lib.check(lib.st2_act_conv_transpose1d_fused_ex_scratch_bytes(B, T, Cin, Cout, k, stride), "fused_t_ex_scratch_bytes")
+    scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev())
+    _lib.check(lib.st2_act_conv_transpose1d_fused_ex(_lib.ptr(xd), _lib.ptr(ad), _lib.ACT[act], C.c_float(slope), _lib.ptr(wd),
+                                                     _lib.ptr(bd), _lib.ptr(rd), _lib.ptr(y), _lib.ptr(hn), _lib.ptr(cn),
+                                                     _lib.ptr(scratch), B, T, Cin, Cout, k, stride, padding, output_padding,
+                                                     int(y16), _lib.PREC[precision], stream()), "act_conv_transpose1d_fused_ex")
+    torch.cuda.synchronize()
+    return y.cpu().numpy(), (None if cn is None else cn.cpu().numpy())
