@@ -252,6 +252,28 @@ ST2_API int st2_har_source(const float* f0, const float* noise, uint64_t seed, c
                    const float* lin_b, float* har, float* frames_scratch, int32_t B, int32_t L2,
                    int32_t upsample_scale, void* stream);
 
+/* generator.noise_convs[i] (hifigan.py:296-303,330) on the harmonic source, as the decoder runs it: har [B,S] ->
+ * y [B,Tout,C] channels-last, Tout = (S + 2*pad - k)/stride + 1, w [C,1,k] (reference layout), bias [C].  y is fp32, or with
+ * y16 fp16 WITHOUT the bias (the decoder's fp16 noise source).  If h [B,2C] is given, coef [B,2,C] receives the AdaIN
+ * coefficients (a = (1+gamma)*rstd, b = beta - mean*a) of the conv output from the kernel's statistics partials, with b
+ * for the tensor as stored (mean taken without the bias when y16).  scratch: st2_noise_conv_scratch_bytes(...) bytes. */
+ST2_API int64_t st2_noise_conv_scratch_bytes(int32_t B, int32_t Tout, int32_t C, int32_t k, int32_t stride);
+ST2_API int st2_noise_conv(const float* har, const float* w, const float* bias, void* y, const float* h, float* coef,
+                   void* scratch, int32_t B, int32_t S, int32_t Tout, int32_t C, int32_t k, int32_t stride, int32_t pad,
+                   int32_t y16, void* stream);
+
+/* Generator tail (hifigan.py:343-345): out [B,S] = tanh(conv_post(snake(x, alpha))), conv_post C -> 1, k = 7, padding 3.
+ * x [B,S,C] channels-last with row pitch ld_x (a multiple of 4), fp32, or fp16 when x16 (needs fast); C a multiple of 4,
+ * <= 64.  w [1,C,7] (reference layout), bias [1], alpha [C].  fast selects __sinf / __fdividef (the 16-bit precisions).
+ * w_scratch: 7*C floats receiving the packed weight. */
+ST2_API int st2_post_hifigan(const void* x, int32_t ld_x, const float* alpha, const float* w, const float* bias, float* out,
+                     float* w_scratch, int32_t B, int32_t S, int32_t C, int32_t fast, int32_t x16, void* stream);
+
+/* All AdaIN fc layers of a decoder in one launch (hifigan.py:18,21): h [B,R] = s [B,K] @ W[R,K]^T + bias [R].
+ * K a multiple of 4, <= 1024. */
+ST2_API int st2_style_fc(const float* s, const float* W, const float* bias, float* h, int32_t B, int32_t R, int32_t K,
+                 void* stream);
+
 /* AdaIN1d + activation (hifigan.py:14-24 with :68 or LeakyReLU) on channels-last
  * x [B,T,C] (pitch ld_x): y = act((1+gamma)*IN(x)+beta), gamma|beta = h[b, 0:C | C:2C].
  * act: 0 none, 1 leaky-relu(slope), 2 snake(alpha[C]).  out_dtype: 0 fp32, 1 bf16, 2 fp16.

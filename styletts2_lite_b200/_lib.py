@@ -99,6 +99,10 @@ SIGNATURES = {
     "st2_length_regulate": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "st2_sinegen_phase": (C.c_int, [_P, _P, _P, _I, _I, _I, _P]),
     "st2_har_source": (C.c_int, [_P, _P, C.c_uint64, _P, _P, _P, _P, _I, _I, _I, _P]),
+    "st2_noise_conv_scratch_bytes": (_L, [_I, _I, _I, _I, _I]),
+    "st2_noise_conv": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "st2_post_hifigan": (C.c_int, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
+    "st2_style_fc": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _P]),
     "st2_adain_scratch_bytes": (_L, [_I, _I, _I]),
     "st2_adain_act": (C.c_int, [_P, _I, _P, _I, _P, _I, C.c_float, _P, _I, _I, _I, _I, _I, _P, _P]),
     "st2_conv1d_scratch_bytes": (_L, [_I, _I, _I, _I, _I, _I]),

@@ -57,6 +57,56 @@ int st2_har_source(const float* f0, const float* noise, uint64_t seed, const flo
                              (cudaStream_t)stream);
 }
 
+// generator.noise_convs[i] + the AdaIN coefficients of its output, as the decoder runs them (decoder.cu, Exec::resblock1)
+static int64_t noise_conv_offsets(int B, int Tout, int C, int k, int stride, int64_t off[2]) {
+    int64_t o = 0;
+    off[0] = o; o += align256((int64_t)k * C * sizeof(float));                                  // packed weight [k][C]
+    off[1] = o; o += align256((int64_t)B * noise_conv_parts(Tout, stride) * C * 8);             // float2 tile partials
+    return o;
+}
+
+int64_t st2_noise_conv_scratch_bytes(int32_t B, int32_t Tout, int32_t C, int32_t k, int32_t stride) {
+    if (B <= 0 || Tout <= 0 || C <= 0 || k <= 0 || stride <= 0) return ST2_ERR_INVALID;
+    int64_t off[2];
+    return noise_conv_offsets(B, Tout, C, k, stride, off);
+}
+
+int st2_noise_conv(const float* har, const float* w, const float* bias, void* y, const float* h, float* coef, void* scratch,
+                   int32_t B, int32_t S, int32_t Tout, int32_t C, int32_t k, int32_t stride, int32_t pad, int32_t y16,
+                   void* stream) {
+    ST2_REQUIRE(har && w && bias && y && scratch && B > 0 && S > 0 && C > 0 && k > 0 && stride > 0 && pad >= 0,
+                "noise_conv: bad argument");
+    ST2_REQUIRE(Tout == (S + 2 * pad - k) / stride + 1 && Tout > 0, "noise_conv: Tout=%d does not match S=%d k=%d stride=%d pad=%d",
+                Tout, S, k, stride, pad);
+    ST2_REQUIRE((h == nullptr) == (coef == nullptr), "noise_conv: h and coef go together");
+    cudaStream_t st = (cudaStream_t)stream;
+    int64_t off[2];
+    noise_conv_offsets(B, Tout, C, k, stride, off);
+    float* wp = (float*)((char*)scratch + off[0]);
+    void* parts = (char*)scratch + off[1];
+    int e = launch_fold_pack(nullptr, w, wp, C, 1, k, 0, st);
+    if (e == ST2_OK) e = launch_noise_conv(har, wp, bias, (float*)y, parts, B, S, Tout, C, k, stride, pad, st, y16 ? 1 : 0);
+    // the partials are of y - bias; the fp16 y is stored without the bias
+    if (e == ST2_OK && h != nullptr)
+        e = launch_adain_coef_f2(parts, noise_conv_parts(Tout, stride), h, 2 * C, 0, coef, B, Tout, C, C, st, y16 ? bias : nullptr,
+                                 bias);
+    return e;
+}
+
+int st2_post_hifigan(const void* x, int32_t ld_x, const float* alpha, const float* w, const float* bias, float* out,
+                     float* w_scratch, int32_t B, int32_t S, int32_t C, int32_t fast, int32_t x16, void* stream) {
+    ST2_REQUIRE(x && alpha && w && bias && out && w_scratch && B > 0 && S > 0 && C > 0 && ld_x >= C, "post_hifigan: bad argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    int e = launch_fold_pack(nullptr, w, w_scratch, 1, C, 7, 0, st);
+    if (e != ST2_OK) return e;
+    return launch_post_hifigan((const float*)x, ld_x, alpha, w_scratch, bias, out, B, S, C, fast ? 1 : 0, st, x16 ? 1 : 0);
+}
+
+int st2_style_fc(const float* s, const float* W, const float* bias, float* h, int32_t B, int32_t R, int32_t K, void* stream) {
+    ST2_REQUIRE(s && W && bias && h && B > 0 && R > 0 && K > 0, "style_fc: bad argument");
+    return launch_style_fc(s, W, bias, h, B, R, K, (cudaStream_t)stream);
+}
+
 int64_t st2_adain_scratch_bytes(int32_t B, int32_t T, int32_t C) {
     if (B <= 0 || T <= 0 || C <= 0) return ST2_ERR_INVALID;
     const int Cpad = (C + 3) / 4 * 4;

@@ -112,6 +112,7 @@ int launch_pool_dw(const float* x, int ld_x, const float* w, const float* bias, 
 int launch_pool_dw16(const float* x, int ld_x, const float* w, const float* bias, void* y, int ld_y, int out_dtype, int B,
                      int T, int Cpad, cudaStream_t st);
 int noise_conv_parts(int Tout, int stride);
+// stats: float2 (sum, sumsq) tile partials of y - bias (the coefficient kernel's stat_shift); y16: y stored as fp16 without the bias
 int launch_noise_conv(const float* har, const float* w, const float* bias, float* y, void* stats, int B, int S, int Tout,
                       int C, int k, int stride, int pad, cudaStream_t st, int y16 = 0);
 int launch_post_hifigan(const float* x, int ld_x, const float* alpha, const float* w, const float* bias,
@@ -209,9 +210,10 @@ bool conv_pipe_supported(const ConvArgs& a);
 int launch_conv_pipe(const ConvArgs& a, const float* coef, int coef_ld, int act, float slope, const float* alpha,
                      void* stats_out, cudaStream_t st);
 int launch_add_vec(float* dst, const float* a, const float* b, int n, cudaStream_t st);
-// x_offset (optional, [C]): the tensor the coefficients will be applied to is stored as x - x_offset[c] (statistics are of x)
+// x_offset (optional, [C]): the tensor the coefficients will be applied to is stored as x - x_offset[c];
+// stat_shift (optional, [C]): the partials are of x - stat_shift[c] (noise_conv: of the conv without its bias)
 int launch_adain_coef_f2(const void* partial, int nparts, const float* h, int ld_h, int h_off, float* coef, int B, int T,
-                         int C, int Cpad, cudaStream_t st, const float* x_offset = nullptr);
+                         int C, int Cpad, cudaStream_t st, const float* x_offset = nullptr, const float* stat_shift = nullptr);
 // 32 / 64-channel stride-1 Snake convs on fp16 stage-private tensors: row-per-thread epilogue, residual through the tensor
 // core, statistics per (CTA, utterance, epilogue warp) (conv_row.cu).  `desc` describes where the partials of an utterance
 // live; launch_adain_coef_row turns them into AdaIN coefficients.

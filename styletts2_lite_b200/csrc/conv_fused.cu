@@ -574,7 +574,8 @@ conv_fused_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
 // (8 independent loads in flight), then a fixed-order tree over the 32 slices -> deterministic.
 __global__ void __launch_bounds__(1024)
 adain_coef_f2_kernel(const float2* __restrict__ partial, int nparts, const float* __restrict__ h, int ld_h, int h_off,
-                     float* __restrict__ coef, int T, int C, int Cpad, const float* __restrict__ x_offset) {
+                     float* __restrict__ coef, int T, int C, int Cpad, const float* __restrict__ x_offset,
+                     const float* __restrict__ stat_shift) {
     __shared__ double ssum[32][33], ssq[32][33];
     pdl_trigger();
     pdl_wait();                 // the partials come from the kernel before this one
@@ -619,15 +620,17 @@ adain_coef_f2_kernel(const float2* __restrict__ partial, int nparts, const float
         const double beta = (double)h[(size_t)b * ld_h + h_off + C + c];
         const double ad = (1.0 + gamma) * rstd;
         a = (float)ad;
+        // partials of x - stat_shift: mean(x) = mean + stat_shift, the variance is that of the partials;
         // stored tensor = x - x_offset: a * x + b = a * (x - x_offset) + (b + a * x_offset)
-        bb = (float)(beta - (mean - (x_offset ? (double)x_offset[c] : 0.0)) * ad);
+        const double d = (stat_shift ? (double)stat_shift[c] : 0.0) - (x_offset ? (double)x_offset[c] : 0.0);
+        bb = (float)(beta - (mean + d) * ad);
     }
     coef[((size_t)b * 2 + 0) * Cpad + c] = a;
     coef[((size_t)b * 2 + 1) * Cpad + c] = bb;
 }
 
 int launch_adain_coef_f2(const void* partial, int nparts, const float* h, int ld_h, int h_off, float* coef, int B, int T,
-                         int C, int Cpad, cudaStream_t st, const float* x_offset) {
+                         int C, int Cpad, cudaStream_t st, const float* x_offset, const float* stat_shift) {
     dim3 grid(cdiv(Cpad, 32), B);
     // programmatic dependent launch for small grids (one-sentence latency): the CTAs may be scheduled while the producing conv
     // drains.  Large batches gain nothing and lose SMs to the next conv's early CTAs (conv_pipe.cu)
@@ -638,7 +641,8 @@ int launch_adain_coef_f2(const void* partial, int nparts, const float* h, int ld
     attr.val.programmaticStreamSerializationAllowed = 1;
     const bool pdl = (int64_t)grid.x * grid.y <= 64;
     cfg.attrs = &attr; cfg.numAttrs = pdl ? 1 : 0;
-    ST2_CUDA_CHECK(cudaLaunchKernelEx(&cfg, adain_coef_f2_kernel, (const float2*)partial, nparts, h, ld_h, h_off, coef, T, C, Cpad, x_offset));
+    ST2_CUDA_CHECK(cudaLaunchKernelEx(&cfg, adain_coef_f2_kernel, (const float2*)partial, nparts, h, ld_h, h_off, coef, T, C, Cpad, x_offset,
+                                      stat_shift));
     ST2_LAUNCH_CHECK();
     return ST2_OK;
 }

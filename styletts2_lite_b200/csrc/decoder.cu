@@ -329,6 +329,7 @@ static int forward_impl(st2_decoder* d, const float* asr, const float* f0, const
                 nc_stats.nparts = noise_conv_parts(Tout, stride);
                 void* stp = E.alloc((int64_t)B * nc_stats.nparts * C * 8);
                 nc_stats.ptr = stp;
+                nc_stats.shift = w.bias;                     // the partials are of the conv without its bias
                 nc_have_stats = true;
                 if (E.live()) {
                     E.chk(launch_noise_conv(har, w.w32, w.bias, nc16 ? (float*)nc16buf : nc, stp, B, S, Tout, C, w.k, stride, pad, st, nc16));

@@ -72,35 +72,42 @@ int launch_f0n_conv(const float* f0, const float* n, const float* wf, const floa
 // ---- all AdaIN fc layers at once: h[B][R] = s[B][K] @ W[R][K]^T + bias[R] ------------------
 // (the 106 nn.Linear(style_dim, 2C) of hifigan.py:18,21).  CTA = 64 utterances x 4 row quads: the style vectors of up to
 // 64 utterances sit in shared memory as [k][b] (conflict-free for consecutive b), every thread owns 4 consecutive output
-// rows of one utterance, reads their weight rows with warp-uniform 128-bit loads and writes one float4.
-static constexpr int kFcB = 64, kFcRq = 4;
+// rows of one utterance, reads their weight rows with warp-uniform 128-bit loads and writes one float4.  Style vectors longer
+// than kFcK are staged kFcK entries at a time (64 KB of shared memory); the summation order stays k = 0..K-1.
+static constexpr int kFcB = 64, kFcRq = 4, kFcK = 256;
 __global__ void __launch_bounds__(kFcB * kFcRq)
 style_fc_kernel(const float* __restrict__ s, const float* __restrict__ W, const float* __restrict__ bias,
                 float* __restrict__ h, int B, int R, int K) {
-    extern __shared__ float ssm[];                    // [K][kFcB]
+    extern __shared__ float ssm[];                    // [min(K, kFcK)][kFcB]
     const int b0 = blockIdx.y * kFcB;
-    for (int i = threadIdx.x; i < K * kFcB; i += kFcB * kFcRq) {
-        const int bb = i / K, k = i - bb * K;         // coalesced read of s, transposed write
-        ssm[k * kFcB + bb] = (b0 + bb < B) ? s[(size_t)(b0 + bb) * K + k] : 0.f;
-    }
-    __syncthreads();
     const int bb = threadIdx.x % kFcB, rq = threadIdx.x / kFcB;
     const int r = (blockIdx.x * kFcRq + rq) * 4;
-    if (r >= R || b0 + bb >= B) return;
+    const bool active = r < R && b0 + bb < B;
     const int nr = min(4, R - r);
     float acc[4] = {0.f, 0.f, 0.f, 0.f};
-    for (int k = 0; k < K; k += 4) {
-        const float s0 = ssm[(k + 0) * kFcB + bb], s1 = ssm[(k + 1) * kFcB + bb], s2 = ssm[(k + 2) * kFcB + bb],
-                    s3 = ssm[(k + 3) * kFcB + bb];
+    for (int k0 = 0; k0 < K; k0 += kFcK) {
+        const int kc = min(kFcK, K - k0);
+        if (k0 > 0) __syncthreads();                  // every thread is done with the previous chunk
+        for (int i = threadIdx.x; i < kc * kFcB; i += kFcB * kFcRq) {
+            const int ib = i / kc, k = i - ib * kc;   // coalesced read of s, transposed write
+            ssm[k * kFcB + ib] = (b0 + ib < B) ? s[(size_t)(b0 + ib) * K + k0 + k] : 0.f;
+        }
+        __syncthreads();
+        if (!active) continue;
+        for (int k = 0; k < kc; k += 4) {
+            const float s0 = ssm[(k + 0) * kFcB + bb], s1 = ssm[(k + 1) * kFcB + bb], s2 = ssm[(k + 2) * kFcB + bb],
+                        s3 = ssm[(k + 3) * kFcB + bb];
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            if (j < nr) {
-                const float4 w = __ldg(reinterpret_cast<const float4*>(W + (size_t)(r + j) * K + k));   // same order as k = 0..K-1
-                acc[j] = fmaf(w.x, s0, acc[j]); acc[j] = fmaf(w.y, s1, acc[j]);
-                acc[j] = fmaf(w.z, s2, acc[j]); acc[j] = fmaf(w.w, s3, acc[j]);
+            for (int j = 0; j < 4; ++j) {
+                if (j < nr) {
+                    const float4 w = __ldg(reinterpret_cast<const float4*>(W + (size_t)(r + j) * K + k0 + k));   // same order as k = 0..K-1
+                    acc[j] = fmaf(w.x, s0, acc[j]); acc[j] = fmaf(w.y, s1, acc[j]);
+                    acc[j] = fmaf(w.z, s2, acc[j]); acc[j] = fmaf(w.w, s3, acc[j]);
+                }
             }
         }
     }
+    if (!active) return;
     float* hp = h + (size_t)(b0 + bb) * R + r;
     for (int j = 0; j < nr; ++j) hp[j] = acc[j] + bias[r + j];
 }
@@ -109,7 +116,7 @@ int launch_style_fc(const float* s, const float* W, const float* bias, float* h,
                     cudaStream_t st) {
     ST2_REQUIRE(K % 4 == 0 && K <= 1024, "style_fc: style_dim %d must be a multiple of 4 and <= 1024", K);
     dim3 grid(cdiv(R, 4 * kFcRq), cdiv(B, kFcB));
-    const size_t smem = (size_t)K * kFcB * sizeof(float);
+    const size_t smem = (size_t)min(K, kFcK) * kFcB * sizeof(float);
     static size_t max_set[kMaxDevices] = {};     // per device (the attribute applies to the current device)
     size_t& ms = max_set[current_device_slot()];
     if (smem > 48 * 1024 && smem > ms) {
@@ -235,9 +242,9 @@ int launch_post_hifigan(const float* x, int ld_x, const float* alpha, const floa
     ST2_REQUIRE(C % 4 == 0 && C <= 64 && ld_x % 4 == 0, "post_hifigan: C=%d ld=%d unsupported", C, ld_x);
     size_t smem = ((size_t)(kPostTile + 6) * (C + 4) + 7 * C) * sizeof(float);
     if (smem > 48 * 1024) {
-        cudaFuncSetAttribute(post_hifigan_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        cudaFuncSetAttribute(post_hifigan_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        cudaFuncSetAttribute(post_hifigan_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        ST2_CUDA_CHECK(cudaFuncSetAttribute(post_hifigan_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        ST2_CUDA_CHECK(cudaFuncSetAttribute(post_hifigan_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        ST2_CUDA_CHECK(cudaFuncSetAttribute(post_hifigan_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     }
     dim3 grid(cdiv(S, kPostTile), B);
     if (x16) post_hifigan_kernel<true, true><<<grid, kPostTile, smem, st>>>(x, ld_x, alpha, w, bias, out, S, C);
@@ -374,7 +381,10 @@ static int nc_tile(int stride) { return stride <= 2 ? 1024 : 256; }
 // input channel every output channel is bias[c] + w[.][c] * har, and a bias larger than the signal would eat the fp16 mantissa
 // that the InstanceNorm behind it then magnifies (measured 4e-2 relative L2 on noise_res.3 with the bias stored).  The consumers
 // add it back: the AdaIN coefficients get the offset (launch_adain_coef_f2) and the residual add of the first iteration has it
-// folded into that conv's bias (decoder.cu).  The statistics still come from the fp32 values with the bias.
+// folded into that conv's bias (decoder.cu).
+// The accumulator and the (sum, sumsq) partials are of y - bias[c]: for the k = 1 conv of the last stage a channel's mean is up
+// to ~500x its std with the reference initialisation, and E[y^2] - mean^2 of fp32 partials of y itself lost 3e-4 of rstd.  The
+// coefficient kernel gets the bias as the statistics' shift; the bias is added only where y is stored as fp32.
 template <bool Y16, int kNcTile>
 __global__ void __launch_bounds__(256)
 noise_conv_kernel(const float* __restrict__ har, const float* __restrict__ w /*[k][C]*/, const float* __restrict__ bias,
@@ -402,7 +412,7 @@ noise_conv_kernel(const float* __restrict__ har, const float* __restrict__ w /*[
     // 4 rows x 4 channels per thread: one 128-bit weight read per tap feeds 16 FMAs
     for (int r = rl; r < kNcTile; r += 4 * rpp) {
         if (t0 + r >= Tout) break;
-        float4 acc[4] = {bv, bv, bv, bv};
+        float4 acc[4] = {};
         const float* hp = sh + r * stride;
         const int hstep = rpp * stride;
         for (int j = 0; j < k; ++j) {
@@ -419,11 +429,12 @@ noise_conv_kernel(const float* __restrict__ har, const float* __restrict__ w /*[
             const int ru = r + u * rpp, t = t0 + ru;
             if (ru >= kNcTile || t >= Tout) break;
             if (Y16) {
-                const __half2 lo = __floats2half2_rn(acc[u].x - bv.x, acc[u].y - bv.y), hi = __floats2half2_rn(acc[u].z - bv.z, acc[u].w - bv.w);
+                const __half2 lo = __floats2half2_rn(acc[u].x, acc[u].y), hi = __floats2half2_rn(acc[u].z, acc[u].w);
                 *reinterpret_cast<uint2*>(reinterpret_cast<__half*>(y) + ((size_t)b * Tout + t) * C + q * 4) =
                     make_uint2(*reinterpret_cast<const uint32_t*>(&lo), *reinterpret_cast<const uint32_t*>(&hi));
             } else {
-                *reinterpret_cast<float4*>(y + ((size_t)b * Tout + t) * C + q * 4) = acc[u];
+                *reinterpret_cast<float4*>(y + ((size_t)b * Tout + t) * C + q * 4) =
+                    make_float4(acc[u].x + bv.x, acc[u].y + bv.y, acc[u].z + bv.z, acc[u].w + bv.w);
             }
             s1[0] += acc[u].x; s1[1] += acc[u].y; s1[2] += acc[u].z; s1[3] += acc[u].w;
             s2[0] = fmaf(acc[u].x, acc[u].x, s2[0]); s2[1] = fmaf(acc[u].y, acc[u].y, s2[1]);

@@ -497,7 +497,8 @@ struct Exec {
     // ---- fused path: statistics references, coefficient kernels, fused conv ---------------------
     // f2: float2 tile partials (conv_pipe / conv_fused epilogues); row: per-(CTA, utterance, warp) partials of conv_row.cu,
     // located by `rd`; neither: double2 slab partials of the standalone statistics pass
-    struct StatRef { const void* ptr; int nparts; bool f2; bool row = false; RowStatsDesc rd = {}; };
+    // shift: the partials are of x - shift[c] (float2 tile partials only)
+    struct StatRef { const void* ptr; int nparts; bool f2; bool row = false; RowStatsDesc rd = {}; const float* shift = nullptr; };
     bool last_row = false;        // did the last conv_fused() run on conv_row.cu (statistics in its layout)?
     RowStatsDesc last_rd = {};
     StatRef produced(const void* buf, int nparts) const {
@@ -521,8 +522,8 @@ struct Exec {
     // x_offset: the tensor is stored as x - x_offset[c] (the bias-free fp16 noise source); only for float2 tile partials
     void coef_from(const StatRef& sr, const AdaINRef* n, int T, int C, int Cpad, const float* x_offset = nullptr) {
         if (!live()) return;
-        if (x_offset != nullptr && (n == nullptr || !sr.f2 || sr.row)) {
-            set_error("coef_from: an input offset needs float2 tile partials");
+        if ((x_offset != nullptr || sr.shift != nullptr) && (n == nullptr || !sr.f2 || sr.row)) {
+            set_error("coef_from: an input offset or statistics shift needs float2 tile partials");
             err = ST2_ERR_STATE;
             return;
         }
@@ -536,7 +537,7 @@ struct Exec {
         else if (sr.row)
             chk(launch_adain_coef_row(sr.ptr, sr.rd, H, d->fc_rows, n->h_off, coef, B, T, C, Cpad, st));
         else
-            chk(launch_adain_coef_f2(sr.ptr, sr.nparts, H, d->fc_rows, n->h_off, coef, B, T, C, Cpad, st, x_offset));
+            chk(launch_adain_coef_f2(sr.ptr, sr.nparts, H, d->fc_rows, n->h_off, coef, B, T, C, Cpad, st, x_offset, sr.shift));
         prof(PC_NORM_COEF, 0, 0);
         coef_ld = Cpad;
     }

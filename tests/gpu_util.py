@@ -264,3 +264,59 @@ def act_conv_transpose1d_fused_ex(x_btc, alpha, act, w, bias, res_btc, h_next, s
                                                      int(y16), _lib.PREC[precision], stream()), "act_conv_transpose1d_fused_ex")
     torch.cuda.synchronize()
     return y.cpu().numpy(), (None if cn is None else cn.cpu().numpy())
+
+
+def har_source_dev(f0_dev, lin_w, lin_b, scale, seed):
+    """st2_har_source with noise drawn on the device (Philox, noise = NULL); f0 and the result stay on the device [B,S]."""
+    lib = _lib.load()
+    B, L2 = f0_dev.shape
+    w, b = to_dev(lin_w.reshape(-1)), to_dev(lin_b.reshape(-1))
+    har = torch.full((B, L2 * scale), float("nan"), device=dev())
+    frames = torch.empty(B, L2, 9, device=dev())
+    _lib.check(lib.st2_har_source(_lib.ptr(f0_dev), None, C.c_uint64(seed), _lib.ptr(w), _lib.ptr(b), _lib.ptr(har),
+                                  _lib.ptr(frames), B, L2, scale, stream()), "har_source")
+    torch.cuda.synchronize()
+    return har
+
+
+def noise_conv(har_dev, w, bias, h, Tout, stride, pad, y16):
+    """st2_noise_conv on a device har [B,S]; w [C,1,k]; h [B,2C] or None.  Returns device tensors (y [B,Tout,C] fp32, or fp16
+    without the bias when y16; coef [B,2,C] or None)."""
+    lib = _lib.load()
+    B, S = har_dev.shape
+    Cc, _, k = w.shape
+    wd, bd = to_dev(w), to_dev(bias)
+    hd = None if h is None else to_dev(h)
+    coef = None if h is None else torch.full((B, 2, Cc), float("nan"), device=dev())
+    y = torch.full((B, Tout, Cc), float("nan"), device=dev(), dtype=torch.float16 if y16 else torch.float32)
+    nbytes = _lib.check(lib.st2_noise_conv_scratch_bytes(B, Tout, Cc, k, stride), "noise_conv_scratch_bytes")
+    scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev())
+    _lib.check(lib.st2_noise_conv(_lib.ptr(har_dev), _lib.ptr(wd), _lib.ptr(bd), _lib.ptr(y), _lib.ptr(hd), _lib.ptr(coef),
+                                  _lib.ptr(scratch), B, S, Tout, Cc, k, stride, pad, int(y16), stream()), "noise_conv")
+    torch.cuda.synchronize()
+    return y, coef
+
+
+def post_hifigan(x_dev, Cc, alpha, w, bias, fast, x16):
+    """st2_post_hifigan on a device x [B,S,ld_x] (fp32, or fp16 when x16) of which the first Cc channels are used; w [1,Cc,7].
+    Returns the device waveform [B,S]."""
+    lib = _lib.load()
+    B, S, ld = x_dev.shape
+    ad, wd, bd = to_dev(alpha.reshape(-1)), to_dev(w), to_dev(bias.reshape(-1))
+    out = torch.full((B, S), float("nan"), device=dev())
+    wsc = torch.empty(7 * Cc, device=dev())
+    _lib.check(lib.st2_post_hifigan(_lib.ptr(x_dev), ld, _lib.ptr(ad), _lib.ptr(wd), _lib.ptr(bd), _lib.ptr(out), _lib.ptr(wsc),
+                                    B, S, Cc, int(fast), int(x16), stream()), "post_hifigan")
+    torch.cuda.synchronize()
+    return out
+
+
+def style_fc(s_dev, W_dev, b_dev):
+    """st2_style_fc: h [B,R] = s [B,K] @ W[R,K]^T + bias, all device tensors."""
+    lib = _lib.load()
+    B, K = s_dev.shape
+    R = W_dev.shape[0]
+    h = torch.full((B, R), float("nan"), device=dev())
+    _lib.check(lib.st2_style_fc(_lib.ptr(s_dev), _lib.ptr(W_dev), _lib.ptr(b_dev), _lib.ptr(h), B, R, K, stream()), "style_fc")
+    torch.cuda.synchronize()
+    return h
