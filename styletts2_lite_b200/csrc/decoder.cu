@@ -308,12 +308,13 @@ static int forward_impl(st2_decoder* d, const float* asr, const float* f0, const
         const bool last = (i + 1 == c.n_stages);
         const int shift = (istft && last) ? 1 : 0;          // ReflectionPad1d((1,0))
         const std::string is = std::to_string(i);
+        const int dtu = E.fmt_for("generator.ups");
+        const int pu = istft ? (ku - u) / 2 : (u / 2 + u % 2);
+        const Exec::StagePlan sp = E.plan_stage(i, Tout, E.fused_args(d->ups[i], dtu, Cin, Tin, C, Tout, u, pu, 1, shift));
+        const int nc16 = sp.src.x16, xu16 = sp.res[0].x16;
         // x_source = noise_res[i](noise_convs[i](har_source), s)
         float* nc = E.allocf((int64_t)B * Tout * C);
-        // noise_convs[i] output = block input of noise_res[i] (read as conv1 input and as the residual of its first iteration):
-        // stored as fp16 when every conv of the block takes it (option fp16_src; statistics still from the fp32 values)
         void* nc16buf = E.alloc((int64_t)B * Tout * C * 2);
-        const int nc16 = (!istft && d->opt_src16 && E.resblock1_x16_ok(d->noise_res[i], Tout, 0)) ? 1 : 0;
         Exec::StatRef nc_stats{nullptr, 0, true};
         bool nc_have_stats = false;
         {
@@ -337,32 +338,22 @@ static int forward_impl(st2_decoder* d, const float* asr, const float* f0, const
                 }
             }
         }
-        E.resblock1(d->noise_res[i], nc16 ? (const float*)nc16buf : nc, nc, Tout, nc, 1.f, 0, nc_have_stats ? &nc_stats : nullptr, nc16,
-                    0, nullptr, 0, nc16 ? d->noise_convs[i].bias : nullptr, nc16 ? d->noise_c2b[i] : nullptr);
+        E.resblock1(d->noise_res[i], sp.src, nc16 ? (const float*)nc16buf : nc, nc, Tout, nc, nc_have_stats ? &nc_stats : nullptr,
+                    nullptr, nc16 ? d->noise_convs[i].bias : nullptr, nc16 ? d->noise_c2b[i] : nullptr);
         // x = ups[i](act(x)) + x_source
-        const int dtu = E.fmt_for("generator.ups");
-        const bool tcu = E.use_tc(d->ups[i], dtu);
-        const int pu = istft ? (ku - u) / 2 : (u / 2 + u % 2);
         float* xu = E.allocf((int64_t)B * Tout * C);
         Exec::StatRef xu_stats{nullptr, 0, true};
-        const bool fuse_u = E.can_fuse(d->ups[i], dtu, Cin, C, u, 1);
-        // The stage input xu = ups(x) + x_source is read six times (input and residual of the first iteration of the three
-        // resblocks): stored as fp16 when the ups conv and all six convs run on the TMA pipeline kernel (fp16_xu = 0: fp32)
-        int xu16 = 0;
-        if (fuse_u && d->opt_xu16 && E.pipe_ok_ups16(d->ups[i], Cin, C, Tin, Tout, u, pu, shift, dtu)) {
-            xu16 = 1;
-            for (int j = 0; j < c.n_kernels; ++j)
-                if (!E.resblock1_x16_ok(d->resblocks[i * c.n_kernels + j], Tout, j > 0 ? 1 : 0)) xu16 = 0;
-        }
-        if (fuse_u) {
+        if (sp.ups_fused) {
             // Snake / LeakyReLU applied on the A-operand path; InstanceNorm statistics of xu from the epilogue
-            xu_stats.nparts = E.fused_parts(d->ups[i], Tout, u, pu, shift);
+            ConvArgs a = sp.ups;
+            xu_stats.nparts = fused_stats_parts(a);
             void* st_xu = E.alloc((int64_t)B * xu_stats.nparts * C * 8);
             xu_stats.ptr = st_xu;
             E.coef_from(Exec::StatRef{nullptr, 0, false}, nullptr, Tin, Cin, Cin);
-            E.conv_fused(d->ups[i], x, Cin, Tin, dtu, istft ? ACT_LRELU : ACT_SNAKE, 0.1f, istft ? nullptr : d->gen_alpha[i], xu, C,
-                         Tout, u, pu, 1, nc, C, 0, 1.f, 0, st_xu, shift, shift, 0, xu16);
+            a.x = x; a.y = xu; a.res = nc;
+            E.conv_fused(a, istft ? ACT_LRELU : ACT_SNAKE, 0.1f, istft ? nullptr : d->gen_alpha[i], st_xu);
         } else {
+            const bool tcu = E.use_tc(d->ups[i], dtu);
             void* xs = E.alloc((int64_t)B * Tin * Cin * (tcu ? 2 : 4));
             if (istft) E.norm_act(x, Cin, Tin, Cin, nullptr, ACT_LRELU, 0.1f, nullptr, xs, Cin, tcu ? dtu : DT_F32);
             else E.norm_act(x, Cin, Tin, Cin, nullptr, ACT_SNAKE, 0.f, d->gen_alpha[i], xs, Cin, tcu ? dtu : DT_F32);
@@ -372,21 +363,11 @@ static int forward_impl(st2_decoder* d, const float* asr, const float* f0, const
         if (xu16) E.tap16("generator.stage" + is + ".in", xu, (int64_t)B * Tout * C);
         else E.tap("generator.stage" + is + ".in", xu, C, (int64_t)B * Tout, C);
         float* run = E.allocf((int64_t)B * Tout * C);
-        // the partial sum over the resblocks of the stage (written by the first, read + written by the middle ones, read by the
-        // last, which writes the fp32 stage output) is kept in fp16 when all their last convs take it (fp16_sum = 0: fp32)
         void* sum16buf = E.alloc((int64_t)B * Tout * C * 2);
-        int sum16 = c.n_kernels >= 2 ? 1 : 0;
-        for (int j = 0; j < c.n_kernels && sum16; ++j)
-            if (!E.resblock1_sum16_ok(d->resblocks[i * c.n_kernels + j], Tout, j == 0 ? 1 : (j + 1 == c.n_kernels ? 3 : 2), xu16)) sum16 = 0;
-        // the last stage's output is only read by conv_post's kernel: fp16 as well when the last block can write it (option fp16_out)
-        out16 = (last && !istft && sum16 && d->opt_out16 &&
-                 E.resblock1_sum16_ok(d->resblocks[i * c.n_kernels + c.n_kernels - 1], Tout, 3, xu16, 1)) ? 1 : 0;
-        for (int j = 0; j < c.n_kernels; ++j) {
-            const bool lastk = (j + 1 == c.n_kernels);
-            E.resblock1(d->resblocks[i * c.n_kernels + j], xu, run, Tout, stage_out[i], lastk ? 1.f / (float)c.n_kernels : 1.f,
-                        j > 0 ? 1 : 0, fuse_u ? &xu_stats : nullptr, xu16, sum16 ? (j == 0 ? 1 : (lastk ? 3 : 2)) : 0, sum16buf,
-                        lastk ? out16 : 0);
-        }
+        for (int j = 0; j < c.n_kernels; ++j)
+            E.resblock1(d->resblocks[i * c.n_kernels + j], sp.res[j], xu, run, Tout, stage_out[i], sp.ups_fused ? &xu_stats : nullptr,
+                        sum16buf);
+        out16 = sp.res[c.n_kernels - 1].dest16;
         if (out16) E.tap16("generator.stage" + is + ".out", stage_out[i], (int64_t)B * Tout * C);
         else E.tap("generator.stage" + is + ".out", stage_out[i], C, (int64_t)B * Tout, C);
         x = stage_out[i];

@@ -78,10 +78,10 @@ struct st2_decoder {
     int64_t last_launches = 0;
     const uint64_t* seed_dev = nullptr;     // optional device-resident Philox seed (st2_decoder_set_seed_buffer)
     bool tc_ok = false;
-    int fp16_storage = 1;                   // st2_decoder_set_option("fp16_storage"): stage-private tensors of the 16-bit paths in fp16
-    // ... and each of the four kinds alone ("fp16_xt", "fp16_run", "fp16_xu", "fp16_sum"; DESIGN.md section 3)
-    int opt_xt16 = 1, opt_run16 = 1, opt_xu16 = 1, opt_sum16 = 1;
-    int opt_src16 = 1, opt_out16 = 1;       // "fp16_src": noise_convs output (input of noise_res); "fp16_out": last stage's output
+    // st2_decoder_set_option("fp16_storage"): stage-private tensors of the 16-bit paths in fp16, and each kind alone ("fp16_xt",
+    // "fp16_run", "fp16_xu", "fp16_sum", "fp16_src", "fp16_out"); read by Exec::plan_stage only
+    int fp16_storage = 1;
+    int opt_xt16 = 1, opt_run16 = 1, opt_xu16 = 1, opt_sum16 = 1, opt_src16 = 1, opt_out16 = 1;
 
     ResBlk1dW encode, decode[4];
     float *f0_w = nullptr, *f0_b = nullptr, *n_w = nullptr, *n_b = nullptr;
@@ -551,71 +551,59 @@ struct Exec {
         a.tap_step = w.transposed ? -1 : dilation;
         return conv_fused_supported(a);
     }
-    int fused_parts(const ConvW& w, int Tout, int stride, int padding, int out_row_shift) {
+    // a fused conv's ConvArgs but for its buffers (x, y, res, acc_src), which the launch fills in: geometry, 16-bit weights,
+    // residual pitch ld_y, epilogue scale 1; shift: the output is written one row down and row 2 mirrored into row 0
+    ConvArgs fused_args(const ConvW& w, int dt, int ld_x, int Tin, int ld_y, int Tout, int stride, int padding, int dilation,
+                        int shift = 0) {
         ConvArgs a;
-        memset(&a, 0, sizeof(a));
-        a.w16_cout_pad = w.cout_pad;
-        a.phases = w.transposed ? stride : 1;
-        a.M = w.transposed ? (Tout - 1 - out_row_shift + padding) / stride + 1 : Tout;
-        return fused_stats_parts(a);
-    }
-    // would launch_conv_fused run this stride-1 conv on the TMA pipeline kernel (conv_pipe.cu) with these storage types?
-    bool pipe_ok(const ConvW& w, int ld_x, int ld_y, int T, int padding, int dilation, bool has_res, int accumulate, int dt,
-                 int x16in, int y16out, int res16 = 0, int acc16 = 0) {
-        ConvArgs a;
-        if (!fill_args(a, w, T, T, 1, padding, dilation, 0)) return false;
-        a.accumulate = accumulate;
-        a.ld_x = ld_x; a.ld_y = ld_y; a.ld_res = ld_y; a.res = has_res ? (const float*)this : nullptr;   // only null-ness matters
+        fill_args(a, w, Tin, Tout, stride, padding, dilation, shift);
+        a.ld_x = ld_x; a.ld_y = ld_y; a.ld_res = ld_y;
+        a.scale = 1.f; a.mirror = shift;
         a.w16 = w.w16[dt]; a.w16_cin_pad = w.cin_pad; a.w16_cout_pad = w.cout_pad; a.fmt16 = dt;
-        a.x16in = x16in; a.y16out = y16out; a.res16 = res16; a.scale = 1.f;
-        if (accumulate && acc16) { a.acc_src = this; a.acc16 = 1; }                                      // only null-ness matters
+        return a;
+    }
+    // would a planned launch run on conv_pipe.cu?  ConvArgs tells a residual (res) and a separate source of the old values
+    // (acc16) by non-null pointers, and a plan is made before its buffers exist (and in the workspace dry run, which has none),
+    // so they are marked with kPlanned here
+    static constexpr float kPlanned = 0.f;
+    bool on_pipe(ConvArgs a, bool res) {
+        if (res) a.res = &kPlanned;
+        if (a.acc16) a.acc_src = &kPlanned;
         return conv_pipe_supported(a);
     }
-    // would launch_conv_fused run this upsampling conv on the TMA pipeline kernel and write a 16-bit output?
-    bool pipe_ok_ups16(const ConvW& w, int ld_x, int ld_y, int Tin, int Tout, int stride, int padding, int shift, int dt) {
-        ConvArgs a;
-        if (shift != 0 || !fill_args(a, w, Tin, Tout, stride, padding, 1, 0)) return false;
-        a.ld_x = ld_x; a.ld_y = ld_y; a.ld_res = ld_y; a.res = (const float*)this;                        // only null-ness matters
-        a.w16 = w.w16[dt]; a.w16_cin_pad = w.cin_pad; a.w16_cout_pad = w.cout_pad; a.fmt16 = dt;
-        a.y16out = 1; a.scale = 1.f;
-        return conv_pipe_supported(a);
-    }
+    // AdaIN of a fused conv's input: the statistics of the input, the AdaIN, and `off` when the input is stored as x - off[c]
+    struct AdaIn { StatRef sr; const AdaINRef* n; const float* off = nullptr; };
     // y = epilogue( conv( act(coef.a * x + coef.b) ) ), statistics of y -> stats_out (float2 partials)
-    void conv_fused(const ConvW& w, const float* x, int ld_x, int Tin, int dt, int act, float slope, const float* alpha,
-                    float* y, int ld_y, int Tout, int stride, int padding, int dilation, const float* res, int ld_res,
-                    int res_shift, float scale, int accumulate, void* stats_out, int out_row_shift = 0, int mirror = 0,
-                    int x16in = 0, int y16out = 0, int res16 = 0, const void* acc_src = nullptr, int acc16 = 0,
-                    const StatRef* in_sr = nullptr, const AdaINRef* in_n = nullptr, const float* in_off = nullptr) {
-        // in_sr / in_n (/ in_off): the statistics and the AdaIN of this conv's input.  When both the producer of the statistics and
-        // this conv run on conv_row.cu the kernel computes its coefficients itself (no launch in between); otherwise the
-        // coefficient kernel is launched here, as coef_from() before the call would
+    void conv_fused(const ConvArgs& a, int act, float slope, const float* alpha, void* stats_out, const AdaIn* in = nullptr) {
+        // with `in`, the coefficients of the input transform come from it: when both the producer of the statistics and this conv
+        // run on conv_row.cu the kernel computes them itself (no launch in between); otherwise the coefficient kernel is launched
+        // here, as coef_from() before the call would
         if (!live()) return;
-        ConvArgs a;
-        if (!fill_args(a, w, Tin, Tout, stride, padding, dilation, out_row_shift)) return;
-        a.res = res; a.ld_res = ld_res; a.res_shift = res_shift;
-        a.y = y; a.ld_y = ld_y;
-        a.scale = scale; a.accumulate = accumulate; a.mirror = mirror;
-        a.x = x; a.ld_x = ld_x; a.w16 = w.w16[dt]; a.w16_cin_pad = w.cin_pad; a.w16_cout_pad = w.cout_pad; a.fmt16 = dt;
-        a.x16in = x16in; a.y16out = y16out; a.res16 = res16; a.acc_src = acc_src; a.acc16 = acc16;
-        // the 32 / 64-channel Snake convs on fp16 tensors run on the row-per-thread kernel (conv_row.cu); its statistics
-        // partials have their own layout, recorded in last_rd for the coefficient kernel
-        const bool row = act == ACT_SNAKE && !w.transposed && conv_row_supported(a);
+        // the kernel, decided once: the 32 / 64-channel Snake convs on fp16 tensors run on the row-per-thread kernel (conv_row.cu;
+        // its statistics partials have their own layout, recorded in last_rd for the coefficient kernel), the rest on conv_pipe.cu
+        // where it takes them, else on conv_fused.cu
+        const int cat = (act == ACT_SNAKE && conv_row_supported(a)) ? PC_CONV_ROW : conv_pipe_supported(a) ? PC_CONV_PIPE : PC_CONV_FUSED;
+        const bool row = cat == PC_CONV_ROW;
         RowCoefSrc src{};
         bool inline_coef = false;
-        if (in_sr != nullptr) {
-            inline_coef = row && in_n != nullptr && in_sr->f2 && in_sr->row && in_off == nullptr && conv_row_inline_coef_ok(a);
-            if (inline_coef) src = RowCoefSrc{in_sr->ptr, in_sr->rd, H, d->fc_rows, in_n->h_off, Tin};
-            else coef_from(*in_sr, in_n, Tin, w.Cin, w.Cin, in_off);
+        if (in != nullptr) {
+            inline_coef = row && in->n != nullptr && in->sr.f2 && in->sr.row && in->off == nullptr && conv_row_inline_coef_ok(a);
+            if (inline_coef) src = RowCoefSrc{in->sr.ptr, in->sr.rd, H, d->fc_rows, in->n->h_off, a.Tin};
+            else coef_from(in->sr, in->n, a.Tin, a.Cin, a.Cin, in->off);
             if (err != ST2_OK) return;
         }
         last_row = row;
         if (row) chk(launch_conv_row(a, coef, coef_ld, act, alpha, stats_out, &last_rd, st, inline_coef ? &src : nullptr));
+        else if (cat == PC_CONV_PIPE) chk(launch_conv_pipe(a, coef, coef_ld, act, slope, alpha, stats_out, st));
         else chk(launch_conv_fused(a, coef, coef_ld, act, slope, alpha, stats_out, st));
-        const double flops = 2.0 * B * (w.transposed ? (double)Tin : (double)(Tout - out_row_shift)) * w.Cin * w.Cout * w.k;
-        const double bytes = (double)B * ((double)w.Cin * Tin * (x16in ? 2 : 4) +
-                                          (double)w.Cout * Tout * ((y16out ? 2 : 4) + (res ? (res16 ? 2 : 4) : 0) + (accumulate ? (acc16 ? 2 : 4) : 0))) +
-                             (double)w.k * w.Cin * w.Cout * 2;
-        prof(last_row ? PC_CONV_ROW : (conv_pipe_supported(a) ? PC_CONV_PIPE : PC_CONV_FUSED), flops, bytes);
+        // algorithmic work as in conv(): k = w_step * ntaps taps; a transposed conv (tap_step -1) counts its Tin input rows
+        const int k = a.w_step * a.ntaps;
+        const double flops = 2.0 * B * (a.tap_step < 0 ? (double)a.Tin : (double)a.Tout) * a.Cin * a.Cout * k;
+        const double bytes = (double)B * ((double)a.Cin * a.Tin * (a.x16in ? 2 : 4) +
+                                          (double)a.Cout * a.Tout * ((a.y16out ? 2 : 4) + (a.res ? (a.res16 ? 2 : 4) : 0) +
+                                                                     (a.accumulate ? (a.acc16 ? 2 : 4) : 0))) +
+                             (double)k * a.Cin * a.Cout * 2;
+        prof(cat, flops, bytes);
     }
 
     // AdainResBlk1d.forward (hifigan.py:400-403).  x [B,T,ld_x] (Cin real channels) -> y [B,T or 2T,ld_y]
@@ -667,107 +655,137 @@ struct Exec {
         off = mark;
     }
 
-    // AdaINResBlock1.forward (hifigan.py:65-74) on x_in [B,T,C]; the running tensor lives in `run`
-    // (may alias x_in for an in-place block); the last iteration writes
-    // dest = (dest_old*accumulate + conv2 + run) * scale.
-    // would resblock1 take its input tensor as fp16 (every conv of the block on the TMA pipeline kernel)?
-    // would the last conv of this block write / accumulate the fp16 partial sum of the stage?
-    //   mode 1: first block of a stage, writes the fp16 sum;  2: middle, fp16 sum in place;  3: last, fp16 sum -> fp32 stage output
-    // dest16 (mode 3 only): the last block writes the stage output as fp16 too
-    bool resblock1_sum16_ok(const ResBlock1W& w, int T, int mode, int x16, int dest16 = 0) {
-        const int C = w.C, dt = fmt_for(w.name);
-        if (!can_fuse(w.c1[0], dt, C, C, 1, 5) || !d->fp16_storage || !d->opt_xt16 || !d->opt_run16 || !d->opt_sum16) return false;
-        for (int j = 0; j < 3; ++j) {        // every conv of the block on the pipeline kernel with the fp16 tensors it will see
-            const int dil = w.dil[j], in16 = (j > 0 || x16) ? 1 : 0;
-            if (!pipe_ok(w.c1[j], C, C, T, (w.k * dil - dil) / 2, dil, false, 0, dt, in16, 1) ||
-                !pipe_ok(w.c2[j], C, C, T, (w.k - 1) / 2, 1, true, (j == 2 && mode > 1) ? 1 : 0, dt, 1, (j < 2 || mode < 3 || dest16) ? 1 : 0, in16,
-                         (j == 2 && mode > 1) ? 1 : 0))
-                return false;
-        }
+    // ---- fp16 storage of a generator stage ---------------------------------------------------------------------------
+    // how a fused AdaINResBlock1 runs (plan_stage): its part in the stage's sum and which of its tensors are stored as fp16
+    struct BlockPlan {
+        bool fused = false;      // on the fused conv kernels; else the coefficient / affine kernels and conv()
+        int accumulate = 0;      // the last conv adds the old values of dest ...
+        float scale = 1.f;       // ... and scales the sum (the last block of a stage: the mean over the blocks)
+        bool xt16 = false;       // the intra-block tensor xt
+        bool run16 = false;      // the running tensor between the iterations (needs xt16)
+        bool x16 = false;        // the block input (needs run16)
+        int sum16 = 0;           // the stage's partial sum, of which the block is the 1 first, 2 middle or 3 last (needs run16)
+        bool dest16 = false;     // dest (needs sum16 == 3)
+    };
+    struct StagePlan {
+        ConvArgs ups;            // generator.ups[i] on the fused path, but for its buffers
+        bool ups_fused = false;
+        BlockPlan src;           // generator.noise_res[i]
+        BlockPlan res[3];        // generator.resblocks[i * 3 + j] (n_kernels is 3, st2_decoder_create)
+    };
+    // convs1[j] (c2 = false) or convs2[j] of fused block w run with plan p, but for its buffers: x, y, the running tensor
+    // (residual of convs2) and, with acc16, the stage's fp16 sum (old values of the last convs2)
+    ConvArgs block_args(const ResBlock1W& w, const BlockPlan& p, int j, bool c2, int T) {
+        const int dil = c2 ? 1 : w.dil[j], run16 = j > 0 ? p.run16 : p.x16;    // the running tensor: the block input at j = 0
+        ConvArgs a = fused_args(c2 ? w.c2[j] : w.c1[j], fmt_for(w.name), w.C, T, w.C, T, 1, (w.k * dil - dil) / 2, dil);
+        a.x16in = c2 ? p.xt16 : run16;
+        a.y16out = !c2 ? p.xt16 : j < 2 ? p.run16 : (p.sum16 != 0 && (p.sum16 < 3 || p.dest16));
+        a.res16 = c2 ? run16 : 0;
+        if (c2 && j == 2) { a.accumulate = p.accumulate; a.scale = p.scale; a.acc16 = p.sum16 > 1 ? 1 : 0; }
+        return a;
+    }
+    bool block_on_pipe(const ResBlock1W& w, const BlockPlan& p, int T) {
+        for (int j = 0; j < 3; ++j)
+            if (!on_pipe(block_args(w, p, j, false, T), false) || !on_pipe(block_args(w, p, j, true, T), true)) return false;
         return true;
     }
-    bool resblock1_x16_ok(const ResBlock1W& w, int T, int accumulate) {
-        const int C = w.C, dt = fmt_for(w.name);
-        if (!can_fuse(w.c1[0], dt, C, C, 1, 5) || !d->fp16_storage || !d->opt_xt16 || !d->opt_run16) return false;
-        for (int j = 0; j < 3; ++j) {
-            const int dil = w.dil[j];
-            if (!pipe_ok(w.c1[j], C, C, T, (w.k * dil - dil) / 2, dil, false, 0, dt, 1, 1) ||
-                !pipe_ok(w.c2[j], C, C, T, (w.k - 1) / 2, 1, true, j == 2 ? accumulate : 0, dt, 1, j < 2, 1))
-                return false;
-        }
-        return true;
+    // The fp16 storage of generator stage i at T rows (DESIGN.md section 3), the only reader of the options fp16_storage and
+    // fp16_*.  A tensor private to the stage is stored as fp16 when every conv that touches it still runs on conv_pipe.cu with
+    // it; its AdaIN statistics still come from the fp32 values in the producing epilogue.  ups: the fused ups conv but for its
+    // buffers and y16out.
+    StagePlan plan_stage(int i, int T, const ConvArgs& ups) {
+        const st2_config& c = d->cfg;
+        const int n = c.n_kernels;
+        const bool istft = c.variant == 1;
+        const ResBlock1W& nr = d->noise_res[i];
+        const ResBlock1W* rb = &d->resblocks[i * n];
+        // (1) xt, conv1's output, read only by conv2's transform: 20 % fewer HBM bytes per iteration for -0.1 dB of SNR
+        // (fp16_xt = 0 turns off every kind)
+        auto block = [&](const ResBlock1W& w, int accumulate, float scale) {
+            BlockPlan p;
+            p.fused = can_fuse(w.c1[0], fmt_for(w.name), w.C, w.C, 1, 5);
+            p.accumulate = accumulate; p.scale = scale;
+            p.xt16 = p.fused && d->fp16_storage && d->opt_xt16;
+            p.xt16 = p.xt16 && block_on_pipe(w, p, T);
+            return p;
+        };
+        // (2) the running tensor between the three iterations (x + conv2 output of iterations 0 and 1, read as the next conv1's
+        // input and conv2's residual; the block output stays fp32): 25 % fewer bytes per block (fp16_run); x16: with an fp16
+        // block input, which needs the statistics of its producer
+        auto takes16 = [&](const ResBlock1W& w, BlockPlan p, bool x16) {
+            p.run16 = p.xt16 && d->opt_run16;
+            p.x16 = p.run16 && x16;
+            return p.run16 && block_on_pipe(w, p, T);
+        };
+        auto input16 = [&](const ResBlock1W& w, BlockPlan& p, bool x16) { p.x16 = x16; p.run16 = x16 || takes16(w, p, false); };
+        StagePlan sp;
+        // (5) the noise_convs output, input of noise_res (conv1 input and residual of its first iteration), stored without its
+        // bias; the istftnet source conv writes no statistics (fp16_src)
+        sp.src = block(nr, 0, 1.f);
+        input16(nr, sp.src, !istft && d->opt_src16 && takes16(nr, sp.src, true));
+        // (3) the stage input xu = ups(x) + x_source, read six times (input and residual of the first iteration of the three
+        // blocks), written by the ups conv (fp16_xu)
+        sp.ups = ups;
+        sp.ups.y16out = 1;
+        sp.ups_fused = can_fuse(d->ups[i], ups.fmt16, ups.ld_x, ups.ld_y, c.upsample_rates[i], 1);
+        bool xu16 = sp.ups_fused && d->opt_xu16 && on_pipe(sp.ups, true);
+        for (int j = 0; j < n; ++j) sp.res[j] = block(rb[j], j > 0 ? 1 : 0, j + 1 == n ? 1.f / (float)n : 1.f);
+        for (int j = 0; j < n; ++j) xu16 = xu16 && takes16(rb[j], sp.res[j], true);
+        sp.ups.y16out = xu16 ? 1 : 0;
+        for (int j = 0; j < n; ++j) input16(rb[j], sp.res[j], xu16);
+        // (4) the partial sum over the blocks, written by the first, read and written in place by the middle ones, read by the
+        // last, which writes the stage output: these accumulate layers sit at their byte floor (fp16_sum)
+        bool sum16 = n >= 2 && d->opt_sum16;
+        for (int j = 0; j < n; ++j) sp.res[j].sum16 = j == 0 ? 1 : (j + 1 == n ? 3 : 2);
+        for (int j = 0; j < n && sum16; ++j) sum16 = sp.res[j].run16 && block_on_pipe(rb[j], sp.res[j], T);
+        for (int j = 0; j < n && !sum16; ++j) sp.res[j].sum16 = 0;
+        // (6) the last stage's output, read only by conv_post's kernel (fp16_out)
+        BlockPlan& lb = sp.res[n - 1];
+        lb.dest16 = sum16 && i + 1 == c.n_stages && !istft && d->opt_out16;
+        lb.dest16 = lb.dest16 && block_on_pipe(rb[n - 1], lb, T);
+        return sp;
     }
-    // sum16 (modes above) with sum16buf: the stage's partial sum lives in fp16 until the last block writes `dest`
-    void resblock1(const ResBlock1W& w, const float* x_in, float* run, int T, float* dest, float scale, int accumulate,
-                   const StatRef* in_stats = nullptr, int x16 = 0, int sum16 = 0, void* sum16buf = nullptr, int dest16 = 0,
-                   const float* x_offset = nullptr, const float* c2b0 = nullptr) {
-        // x_offset / c2b0: x_in is stored as x - x_offset[c]; c2b0 = c2[0].bias + x_offset puts it back in the residual add
+
+    // AdaINResBlock1.forward (hifigan.py:65-74) on x_in [B,T,C] run with plan p; the running tensor lives in `run` (may alias
+    // x_in for an in-place block); the last iteration writes dest = (dest_old*accumulate + conv2 + run) * scale, through the
+    // stage's fp16 partial sum sum16buf when p.sum16.  in_stats: statistics of x_in from its producer (else a standalone pass).
+    // x_offset / c2b0: x_in is stored as x - x_offset[c]; c2b0 = c2[0].bias + x_offset puts it back in the residual add
+    void resblock1(const ResBlock1W& w, const BlockPlan& p, const float* x_in, float* run, int T, float* dest,
+                   const StatRef* in_stats = nullptr, void* sum16buf = nullptr, const float* x_offset = nullptr,
+                   const float* c2b0 = nullptr) {
         const int64_t mark = off;
         const int C = w.C;
         const int dt = fmt_for(w.name);
-        if (can_fuse(w.c1[0], dt, C, C, 1, 5)) {
+        if (p.fused) {
             // fused: 2 tiny coefficient kernels + 2 fused convs per iteration; AdaIN statistics come from the
             // producing conv's epilogue (or from in_stats for the block input)
-            const int nparts = fused_parts(w.c1[0], T, 1, 0, 0);
+            const int nparts = fused_stats_parts(block_args(w, p, 0, false, T));
             int64_t st_bytes = (int64_t)B * nparts * C * 8;
             if ((C == 32 || C == 64) && conv_row_stats_bytes(B, T, C) > st_bytes) st_bytes = conv_row_stats_bytes(B, T, C);
             void* st_xt = alloc(st_bytes);
             void* st_run = alloc(st_bytes);
-            // the intra-block tensor xt (conv1 output, only consumed by conv2's transform) is stored as fp16 when both convs
-            // run on the TMA pipeline kernel: 20 % fewer HBM bytes per iteration for -0.1 dB of SNR (its statistics still come
-            // from the fp32 values in the epilogue).  option fp16_xt = 0 keeps it fp32.
-            int xt16 = (d->fp16_storage && d->opt_xt16) ? 1 : 0;
-            for (int j = 0; j < 3 && xt16; ++j) {
-                const int dil = w.dil[j];
-                if (!pipe_ok(w.c1[j], C, C, T, (w.k * dil - dil) / 2, dil, false, 0, dt, 0, 1) ||
-                    !pipe_ok(w.c2[j], C, C, T, (w.k - 1) / 2, 1, true, j == 2 ? accumulate : 0, dt, 1, 0))
-                    xt16 = 0;
-            }
             float* xt = (float*)alloc((int64_t)B * T * C * 4);      // sized for fp32 (the dry run must not depend on the device)
-            // The running tensor between the three iterations (x + conv2 output of iterations 0 and 1; read as conv1's
-            // input and conv2's residual by the next iteration) is private to the block: stored as fp16 as well when every
-            // conv of the block takes it (25 % fewer HBM bytes per block; AdaIN statistics still come from the fp32 values in
-            // the epilogue, the stage output the last iteration writes stays fp32).  option fp16_run = 0 keeps it fp32.
-            int run16 = (xt16 && d->opt_run16) ? 1 : 0;
-            for (int j = 0; j < 3 && run16; ++j) {
-                const int dil = w.dil[j];
-                if (!pipe_ok(w.c1[j], C, C, T, (w.k * dil - dil) / 2, dil, false, 0, dt, j > 0 || x16, 1) ||
-                    !pipe_ok(w.c2[j], C, C, T, (w.k - 1) / 2, 1, true, j == 2 ? accumulate : 0, dt, 1, j < 2, j > 0 || x16))
-                    run16 = 0;
-            }
             void* r16buf = alloc((int64_t)B * T * C * 2);           // allocated either way: same workspace on every device
-            if (sum16 && !run16 && err == ST2_OK) {                  // the caller asks resblock1_sum16_ok first
-                set_error("resblock1: the fp16 stage sum needs the fp16 running-tensor path");
-                err = ST2_ERR_STATE;
-            }
-            if (x16 && !(run16 && in_stats) && err == ST2_OK) {      // the caller asks resblock1_x16_ok first
-                set_error("resblock1: fp16 block input needs the fp16 running-tensor path and producer statistics");
-                err = ST2_ERR_STATE;
-            }
             StatRef cur_st = in_stats ? *in_stats : stats_standalone(x_in, C, T, C);
             const float* cur = x_in;
-            int cur16 = x16;
             for (int j = 0; j < 3; ++j) {
-                const int dil = w.dil[j];
-                const StatRef sr1 = cur_st;
-                conv_fused(w.c1[j], cur, C, T, dt, ACT_SNAKE, 0.f, w.alpha1[j], xt, C, T, 1, (w.k * dil - dil) / 2, dil, nullptr,
-                           0, 0, 1.f, 0, st_xt, 0, 0, cur16, xt16, 0, nullptr, 0, &sr1, &w.n1[j], j == 0 ? x_offset : nullptr);
-                if (!xt16) tap(w.name + ".convs1." + std::to_string(j), xt, C, (int64_t)B * T, C);
-                else tap16(w.name + ".convs1." + std::to_string(j), xt, (int64_t)B * T * C);
-                const StatRef sr2 = produced(st_xt, nparts);
                 const bool last = (j == 2);
-                const bool s16 = last && sum16 != 0 && run16;                     // the caller asked resblock1_sum16_ok first
-                const int out16 = ((run16 && !last) || (s16 && (sum16 < 3 || dest16))) ? 1 : 0;
-                float* out = last ? ((s16 && sum16 < 3) ? (float*)sum16buf : dest) : (out16 ? (float*)r16buf : run);
-                ConvW c2 = w.c2[j];
-                if (j == 0 && x_offset != nullptr) c2.bias = const_cast<float*>(c2b0);
-                conv_fused(c2, xt, C, T, dt, ACT_SNAKE, 0.f, w.alpha2[j], out, C, T, 1, (w.k - 1) / 2, 1, cur, C, 0,
-                           last ? scale : 1.f, last ? accumulate : 0, last ? nullptr : st_run, 0, 0, xt16, out16, cur16,
-                           (s16 && sum16 > 1) ? sum16buf : nullptr, (s16 && sum16 > 1) ? 1 : 0, &sr2, &w.n2[j]);
-                if (out16 && !(last && dest16)) tap16(w.name + ".iter" + std::to_string(j), out, (int64_t)B * T * C);
-                else if (!last || (!accumulate && scale == 1.f)) tap(w.name + ".iter" + std::to_string(j), out, C, (int64_t)B * T, C);
+                ConvArgs a1 = block_args(w, p, j, false, T);
+                a1.x = cur; a1.y = xt;
+                const AdaIn in1{cur_st, &w.n1[j], j == 0 ? x_offset : nullptr};
+                conv_fused(a1, ACT_SNAKE, 0.f, w.alpha1[j], st_xt, &in1);
+                if (!p.xt16) tap(w.name + ".convs1." + std::to_string(j), xt, C, (int64_t)B * T, C);
+                else tap16(w.name + ".convs1." + std::to_string(j), xt, (int64_t)B * T * C);
+                ConvArgs a2 = block_args(w, p, j, true, T);
+                float* out = last ? ((p.sum16 == 1 || p.sum16 == 2) ? (float*)sum16buf : dest) : (p.run16 ? (float*)r16buf : run);
+                a2.x = xt; a2.y = out; a2.res = cur;
+                if (a2.acc16) a2.acc_src = sum16buf;
+                if (j == 0 && x_offset != nullptr) a2.bias = c2b0;
+                const AdaIn in2{produced(st_xt, nparts), &w.n2[j]};
+                conv_fused(a2, ACT_SNAKE, 0.f, w.alpha2[j], last ? nullptr : st_run, &in2);
+                if (a2.y16out && !(last && p.dest16)) tap16(w.name + ".iter" + std::to_string(j), out, (int64_t)B * T * C);
+                else if (!last || (!p.accumulate && p.scale == 1.f)) tap(w.name + ".iter" + std::to_string(j), out, C, (int64_t)B * T, C);
                 cur = out;
-                cur16 = out16;
                 cur_st = produced(st_run, nparts);
             }
             off = mark;
@@ -786,9 +804,9 @@ struct Exec {
             norm_act(xt, C, T, C, &w.n2[j], ACT_SNAKE, 0.f, w.alpha2[j], xa, C, dta);
             const bool last = (j == 2);
             float* out = last ? dest : run;
-            conv(w.c2[j], xa, C, T, dta, out, C, T, 1, (w.k - 1) / 2, 1, cur, C, 0, last ? scale : 1.f,
-                 last ? accumulate : 0);
-            if (!last || (!accumulate && scale == 1.f)) tap(w.name + ".iter" + std::to_string(j), out, C, (int64_t)B * T, C);
+            conv(w.c2[j], xa, C, T, dta, out, C, T, 1, (w.k - 1) / 2, 1, cur, C, 0, last ? p.scale : 1.f,
+                 last ? p.accumulate : 0);
+            if (!last || (!p.accumulate && p.scale == 1.f)) tap(w.name + ".iter" + std::to_string(j), out, C, (int64_t)B * T, C);
             cur = out;
         }
         off = mark;
